@@ -2,6 +2,7 @@
 """bench.py -- benchmark of the ScaML-GP hot path (BASELINE.json metric, configs 3 / 4 / 5).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--metric evals|posterior]
+                  [--dump-outputs DIR]
 
 Headline (`--metric evals`, the default): config 3 of BASELINE.json -- **4096 meta-tasks in total** x n=256 x d=6,
 R=6 hyper-parameter rows per task (1 warm start + 5 prior samples, reference scamlgp/utils.py:173-203).  A "step" is
@@ -24,6 +25,11 @@ HBM-bound), `conditioned` and `acq_grad` (target-GP conditioning and analytic ca
 `--impl reference` times the reference's CPU path (the oracle restatement of its botorch/gpytorch arithmetic -- those
 packages cannot be installed here, SURVEY 8c) on the box's host cores in the reference's own parallel style: one
 single-threaded process per core over disjoint task slices (scamlgp/benchmarking/local_runner.py:107-108,174-181).
+
+`--dump-outputs DIR` writes what the last timed step of the printed metric computed, gathered over all ranks, as
+DIR/<name>.npy in float64: for `evals` lml [4096, 6], grad [4096, 6, 8], info [4096, 6] (0 = factorised) and
+stats [2] (sum of LML, failed rows); for `posterior` mean and var [candidates] (8 MB each at 1 Mi candidates).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -379,6 +385,14 @@ def measured_hbm_gbs():
         return 6550.0, "fallback of /opt/skills/guides/B200_PROFILING.md (no MEASURED_PEAKS.json)"
 
 
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.detach().cpu().double().numpy())
+
+
 def run_ours(args) -> None:
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -444,6 +458,16 @@ def run_ours(args) -> None:
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize(device)
+
+    dumps = {}  # --dump-outputs: the last timed step's results, copied before later legs reuse the buffers
+
+    def all_tasks(t):
+        """This rank's block of tasks -> all M tasks on rank 0, None on the others (blocks may differ in size)."""
+        if world == 1:
+            return t.clone()
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object(t.cpu(), parts, dst=0)
+        return torch.cat(parts) if rank == 0 else None
 
     def reduce_stats(l, i):
         # the scalar LML / failure-count reduction of a sharded fit (SURVEY 8e): local sums, one all_reduce
@@ -537,8 +561,8 @@ def run_ours(args) -> None:
     def posterior_bench(full_size: bool):
         """Weighted ScaML-GP prior prediction (mean + variance reduced over the rank's block of the 4096 fitted
         base GPs inside the kernel, then ONE all_reduce(sum) over [2, B]) at B replicated candidates; one "point" =
-        one (task, candidate) pair.  Config 5 asks for B = 1 Mi: that is one timed step here (warm-up on 3 slices of
-        2 x 148 x 64 candidates)."""
+        one (task, candidate) pair.  Config 5 asks for B = 1 Mi: each timed step covers all of them (warm-up on 3
+        slices of 2 x 148 x 64 candidates)."""
         B_SLICE = 2 * 148 * 64
         B_STEP = C5_CANDIDATES if full_size else B_SLICE
         fs = eng.factorize(batch, thd[:, 0].contiguous(), spec)
@@ -570,10 +594,15 @@ def run_ours(args) -> None:
 
         for _ in range(3):  # warm-up slices
             predict(Xc[:B_SLICE], part)
-        psteps = (1 if world == 1 else 2) if full_size else max(2, min(args.steps, 4))
+        if args.metric == "posterior":  # the printed metric: --steps timed steps, resident and end to end
+            psteps = esteps = args.steps
+        else:  # a side leg of the evals line
+            psteps = (1 if world == 1 else 2) if full_size else max(2, min(args.steps, 4))
+            esteps = 1 if full_size else psteps
         ms_r, nl = timed(step_res, psteps, 0 if full_size else 1)
+        if args.dump_outputs and args.metric == "posterior":  # `part` holds the prediction over all tasks
+            dumps.update(mean=part[0].clone(), var=part[1].clone())
         ms_k = timed(step_kernel_only, 1, 0)[0] if world > 1 else ms_r / psteps  # per step, kernel alone
-        esteps = 1 if full_size else psteps
         ms_e, _ = timed(step_e2e, esteps, 0)  # leaves the all-reduced prediction in `part`
         finite = bool(torch.isfinite(part).all() and (part[1] > 0).all())
         # replicated-candidate check: the all-reduced prediction equals ONE GPU holding all 4096 tasks (first 512
@@ -758,6 +787,8 @@ def run_ours(args) -> None:
                          "data": "synthetic", "clocks": clocks})
             if cpu_posterior is not None:
                 post["cpu_baseline"] = cpu_posterior
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, dumps)
             print(json.dumps(post), flush=True)
         if world > 1:
             dist.destroy_process_group()
@@ -769,6 +800,8 @@ def run_ours(args) -> None:
         sampler.start()
     ms_res, launches = timed(step_resident, args.steps, max(3, args.warmup))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dumps.update(lml=all_tasks(lml), grad=all_tasks(grad), info=all_tasks(info), stats=stats.clone())
     e2e_steps = max(2, min(args.steps, 5))
     ms_e2e, _ = timed(step_e2e, e2e_steps, 2)
     ok = int((info == 0).all())
@@ -857,6 +890,8 @@ def run_ours(args) -> None:
         if cpu_baseline is not None:
             line["cpu_baseline"] = cpu_baseline
             line["cpu_baseline_sequential"] = cpu_sequential
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -865,7 +900,9 @@ def run_ours(args) -> None:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of the printed metric (default 20; for --impl ours --metric posterior 1, 2 on "
+                         "several GPUs, 4 with --quick)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--metric", choices=["evals", "posterior"], default="evals",
@@ -875,7 +912,19 @@ def main():
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling side measurement (N > 1)")
     ap.add_argument("--quick", action="store_true",
                     help="profiling runs: posterior leg on a 18944-candidate slice instead of 1 Mi, no config-4 leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps is None:
+        if args.impl == "ours" and args.metric == "posterior":
+            # one full-size step (4096 tasks x 1 Mi candidates) takes about 12 s on one B200 at a 1000 W power limit
+            args.steps = 4 if args.quick else (1 if int(os.environ.get("WORLD_SIZE", "1")) == 1 else 2)
+        else:
+            args.steps = 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
