@@ -240,6 +240,34 @@ int scaml_posterior_grad(const double* X, const int32_t* n_valid, const double* 
                          double s_all, double* dmean, double* dvar, void* workspace, size_t workspace_bytes, int M,
                          int n_max, int d, int B, int n_t, int kernel, int kernel_t, void* stream);
 
+/* Joint posterior of q-point blocks (batch acquisition, q > 1: botorch's optimize_acqf over q candidates jointly, by
+ * autograd through `ScaMLGP.forward`, eval branch, reference scamlgp/model.py:364-375).  Xc [B][d] holds B / q blocks
+ * of q consecutive points, 1 <= q <= 16, B % q == 0, B <= 128 per call.  U is the output of scaml_cond_prepare_pruned
+ * at Xc (as for scaml_posterior_grad); with c_m = w_m^2 ystd_m^2:
+ *   scaml_qblock_cov : weighted prior block of every block, cov [B / q][q][q],
+ *                        cov[b][i][j] = sum_m c_m ( s_m kappa_m(x_i, x_j) - k*_m(x_i)^T K_m^-1 k*_m(x_j) )
+ *                      (exactly symmetric; its diagonal is the variance of scaml_predict_weighted).  U is read only.
+ *                      The conditioning on the target points, Sigma = cov + s_all^2 (s_t kappa_t(x_i, x_j) -
+ *                      k_s(x_i)^T beta(x_j)), is n_t-dimensional and left to the caller.
+ *   scaml_qblock_vjp : vector-Jacobian product of the conditioned posterior (mean [B], Sigma [B / q][q][q], the
+ *                      quantities of scaml_target_posterior_beta / scaml_qblock_cov): given g_mean [B] = da/dmean and
+ *                      g_cov [B / q][q][q] = da/dSigma, dX [B][d] = da/dXc.  Same inputs as scaml_posterior_grad
+ *                      (beta from scaml_target_posterior_beta; NULL Xt, A, alpha_t, beta for n_t = 0) plus theta_t,
+ *                      which is required for every n_t (s_t kappa_t(x_i, x_j) is part of Sigma).  U is CONSUMED.
+ *                      kernel_t = 0..3 (no task-sharded partial sums).
+ * Tasks with w == 0 are skipped; every sum over tasks runs in a fixed order (deterministic). */
+size_t scaml_qblock_cov_workspace_bytes(int M, int B, int q);
+int scaml_qblock_cov(const double* X, const int32_t* n_valid, const double* theta, const double* ystd,
+                     const double* w, const double* Xc, const double* U, double* cov, void* workspace,
+                     size_t workspace_bytes, int M, int n_max, int d, int B, int q, int kernel, void* stream);
+size_t scaml_qblock_vjp_workspace_bytes(int M, int n_max, int d, int B, int n_t);
+int scaml_qblock_vjp(const double* X, const int32_t* n_valid, const double* theta, const double* alpha,
+                     const double* ystd, const double* w, const double* Xc, double* U, const double* Xt,
+                     const double* A, const double* alpha_t, const double* beta, const double* theta_t,
+                     double s_all, const double* g_mean, const double* g_cov, double* dX, void* workspace,
+                     size_t workspace_bytes, int M, int n_max, int d, int B, int q, int n_t, int kernel,
+                     int kernel_t, void* stream);
+
 /* The same quantities as scaml_predict_conditioned (weighted prior mean [B], variance [B], cross-covariance with the
  * target inputs [B][n_t]; reference scamlgp/model.py:364-375, q = 1) computed from U = K_m^-1 K_m(X_m, Xc) instead of a
  * second pass over the packed factors: mean = sum w (ybar + ystd k*^T alpha), var = sum c (s - k*^T u),

@@ -111,6 +111,10 @@ EXPORTED_SYMBOLS = (
     "scaml_target_posterior_beta",
     "scaml_posterior_grad_workspace_bytes",
     "scaml_posterior_grad",
+    "scaml_qblock_cov_workspace_bytes",
+    "scaml_qblock_cov",
+    "scaml_qblock_vjp_workspace_bytes",
+    "scaml_qblock_vjp",
     "scaml_cond_prepare_pruned",
     "scaml_cond_combine_task_splits",
     "scaml_posterior_values_from_u_workspace_bytes",
@@ -180,6 +184,12 @@ class ScamlLib:
         L.scaml_posterior_grad_workspace_bytes.restype = sz
         L.scaml_posterior_grad_workspace_bytes.argtypes = [i32, i32, i32, i32]
         L.scaml_posterior_grad.argtypes = [vp] * 13 + [dbl, vp, vp, vp, sz] + [i32] * 7 + [vp]
+        L.scaml_qblock_cov_workspace_bytes.restype = sz
+        L.scaml_qblock_cov_workspace_bytes.argtypes = [i32, i32, i32]
+        L.scaml_qblock_cov.argtypes = [vp] * 9 + [sz] + [i32] * 6 + [vp]
+        L.scaml_qblock_vjp_workspace_bytes.restype = sz
+        L.scaml_qblock_vjp_workspace_bytes.argtypes = [i32] * 5
+        L.scaml_qblock_vjp.argtypes = [vp] * 13 + [dbl] + [vp] * 4 + [sz] + [i32] * 8 + [vp]
         L.scaml_posterior_values_from_u_workspace_bytes.restype = sz
         L.scaml_posterior_values_from_u_workspace_bytes.argtypes = [i32, i32, i32]
         L.scaml_posterior_values_from_u.argtypes = [vp] * 15 + [sz] + [i32] * 6 + [vp]
@@ -287,6 +297,22 @@ class ScamlLib:
         _check(self.lib.scaml_posterior_grad(X, n_valid, theta, alpha, ystd, w, Xc, U, Xt, A, alpha_t, beta, theta_t,
                                              float(s_all), dmean, dvar, ws, ws_bytes, M, n_max, d, B, n_t, kernel,
                                              kernel_t, stream), "scaml_posterior_grad")
+
+    def qblock_cov_workspace_bytes(self, M: int, B: int, q: int) -> int:
+        return int(self.lib.scaml_qblock_cov_workspace_bytes(M, B, q))
+
+    def qblock_cov(self, X, n_valid, theta, ystd, w, Xc, U, cov, ws, ws_bytes, M, n_max, d, B, q, kernel, stream=0):
+        _check(self.lib.scaml_qblock_cov(X, n_valid, theta, ystd, w, Xc, U, cov, ws, ws_bytes, M, n_max, d, B, q, kernel,
+                                         stream), "scaml_qblock_cov")
+
+    def qblock_vjp_workspace_bytes(self, M: int, n_max: int, d: int, B: int, n_t: int) -> int:
+        return int(self.lib.scaml_qblock_vjp_workspace_bytes(M, n_max, d, B, n_t))
+
+    def qblock_vjp(self, X, n_valid, theta, alpha, ystd, w, Xc, U, Xt, A, alpha_t, beta, theta_t, s_all, g_mean, g_cov,
+                   dX, ws, ws_bytes, M, n_max, d, B, q, n_t, kernel, kernel_t, stream=0):
+        _check(self.lib.scaml_qblock_vjp(X, n_valid, theta, alpha, ystd, w, Xc, U, Xt, A, alpha_t, beta, theta_t,
+                                         float(s_all), g_mean, g_cov, dX, ws, ws_bytes, M, n_max, d, B, q, n_t, kernel,
+                                         kernel_t, stream), "scaml_qblock_vjp")
 
     def posterior_values_from_u_workspace_bytes(self, M: int, B: int, n_t: int) -> int:
         return int(self.lib.scaml_posterior_values_from_u_workspace_bytes(M, B, n_t))

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 CUDA_LIB = os.path.join(CSRC, "libscaml_b200.so")
 
 CUDA_SOURCES = ["scaml_capi.cu", "scaml_microbench.cu"]
-HEADERS = ["scaml_device.cuh", "scaml_fit.cuh", "scaml_fit8.cuh", "scaml_kmat.cuh", "scaml_predict.cuh", "scaml_cond.cuh", "scaml_cross.cuh", "scaml_target.cuh", "scaml_lbfgs.cuh", "scaml_grad.cuh", "scaml_gradval.cuh",
+HEADERS = ["scaml_device.cuh", "scaml_fit.cuh", "scaml_fit8.cuh", "scaml_kmat.cuh", "scaml_predict.cuh", "scaml_cond.cuh", "scaml_cross.cuh", "scaml_target.cuh", "scaml_lbfgs.cuh", "scaml_grad.cuh", "scaml_gradval.cuh", "scaml_qblock.cuh",
            os.path.join("emu", "cuda_emu.h"), os.path.join("..", "..", "include", "scaml_b200.h")]
 
 NVCC_COMPILE_FLAGS = [

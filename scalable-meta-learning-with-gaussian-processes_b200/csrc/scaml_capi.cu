@@ -6,7 +6,7 @@
 //   part 0  fit kernel (4-warp), limits / version / workspace queries
 //   part 1  fit kernel (8-warp)
 //   part 2  kernel matrix, prediction, conditioning, values-from-U
-//   part 3  cross blocks, target GP, L-BFGS update, candidate gradients
+//   part 3  cross blocks, target GP, L-BFGS update, candidate gradients, q-point blocks
 #ifndef SCAML_PART
 #define SCAML_PART (-1)
 #endif
@@ -27,6 +27,7 @@
 #include "scaml_target.cuh"
 #include "scaml_lbfgs.cuh"
 #include "scaml_grad.cuh"
+#include "scaml_qblock.cuh"
 #endif
 #include "scaml_device.cuh"
 
@@ -511,6 +512,73 @@ int scaml_posterior_grad(const double* X, const int32_t* n_valid, const double* 
   p.aal = p.part + (size_t)p.nsplit * (size_t)B * 2 * (size_t)d;
   p.kernel_t = kernel_t;
   return scaml::launch_posterior_grad(p, kernel, num_sms(), stream);
+}
+
+size_t scaml_qblock_cov_workspace_bytes(int M, int B, int q) {
+  if (M <= 0 || B <= 0 || q <= 0) return 0;
+  const int ntile = (B + 31) / 32;
+  return sizeof(double) * (size_t)scaml::grad_nsplit(M, ntile, num_sms()) * (size_t)B * (size_t)q;
+}
+
+int scaml_qblock_cov(const double* X, const int32_t* n_valid, const double* theta, const double* ystd, const double* w,
+                     const double* Xc, const double* U, double* cov, void* workspace, size_t workspace_bytes, int M,
+                     int n_max, int d, int B, int q, int kernel, void* stream) {
+  if (!X || !theta || !ystd || !w || !Xc || !U || !cov || !workspace) return SCAML_E_ARG;
+  if (M <= 0 || n_max <= 0 || d <= 0 || B <= 0 || q <= 0 || B % q != 0 || kernel < 0 || kernel > 3) return SCAML_E_ARG;
+  if (d > scaml::kMaxP - 2 || B > 128 || q > scaml::kQMax) return SCAML_E_UNSUPPORTED;
+  if (workspace_bytes < scaml_qblock_cov_workspace_bytes(M, B, q)) return SCAML_E_WORKSPACE;
+  scaml::QBlockCovParams p{};
+  p.X = X, p.n_valid = n_valid, p.theta = theta, p.ystd = ystd, p.w = w, p.Xc = Xc, p.U = U, p.cov = cov;
+  p.M = M, p.n_max = n_max, p.n_pad = pad64(n_max), p.d = d, p.B = B, p.B_p = scaml::cond_ntp(B), p.q = q;
+  p.ntile = (B + 31) / 32;
+  p.nsplit = scaml::grad_nsplit(M, p.ntile, num_sms());
+  p.part = static_cast<double*>(workspace);
+  return scaml::launch_qblock_cov(p, kernel, num_sms(), stream);
+}
+
+size_t scaml_qblock_vjp_workspace_bytes(int M, int n_max, int d, int B, int n_t) {
+  if (M <= 0 || n_max <= 0 || d <= 0 || B <= 0 || n_t < 0) return 0;
+  return scaml_posterior_grad_workspace_bytes(M, n_max, d, B) +
+         sizeof(double) * ((size_t)2 * B * d + (size_t)B * scaml::cond_ntp(n_t));
+}
+
+int scaml_qblock_vjp(const double* X, const int32_t* n_valid, const double* theta, const double* alpha,
+                     const double* ystd, const double* w, const double* Xc, double* U, const double* Xt, const double* A,
+                     const double* alpha_t, const double* beta, const double* theta_t, double s_all,
+                     const double* g_mean, const double* g_cov, double* dX, void* workspace, size_t workspace_bytes,
+                     int M, int n_max, int d, int B, int q, int n_t, int kernel, int kernel_t, void* stream) {
+  if (!X || !theta || !alpha || !ystd || !w || !Xc || !U || !theta_t || !g_mean || !g_cov || !dX || !workspace)
+    return SCAML_E_ARG;
+  if (M <= 0 || n_max <= 0 || d <= 0 || B <= 0 || q <= 0 || B % q != 0 || n_t < 0 || kernel < 0 || kernel > 3 ||
+      kernel_t < 0 || kernel_t > 3)
+    return SCAML_E_ARG;
+  if (n_t > 0 && (!Xt || !A || !alpha_t || !beta || !(s_all > 0.0))) return SCAML_E_ARG;
+  if (d > scaml::kMaxP - 2 || n_t > 128 || B > 128 || q > scaml::kQMax) return SCAML_E_UNSUPPORTED;
+  if (workspace_bytes < scaml_qblock_vjp_workspace_bytes(M, n_max, d, B, n_t)) return SCAML_E_WORKSPACE;
+  const int n_tp = n_t > 0 ? scaml::cond_ntp(n_t) : 0;
+  double* ws = static_cast<double*>(workspace);
+  double* dmean = ws + scaml_posterior_grad_workspace_bytes(M, n_max, d, B) / sizeof(double);
+  double* dvar = dmean + (size_t)B * d;
+  double* beta_f = dvar + (size_t)B * d;
+  scaml::GradParams g{};
+  g.X = X, g.n_valid = n_valid, g.theta = theta, g.alpha = alpha, g.ystd = ystd, g.w = w, g.Xc = Xc, g.U = U;
+  g.Xt = Xt, g.A = A, g.alpha_t = alpha_t, g.beta = beta_f, g.theta_t = theta_t;
+  g.dmean = dmean, g.dvar = dvar;
+  g.s_all = n_t > 0 ? s_all : 1.0;
+  g.M = M, g.n_max = n_max, g.n_pad = pad64(n_max), g.d = d, g.B = B, g.B_p = scaml::cond_ntp(B);
+  g.n_t = n_t, g.n_tp = n_tp;
+  g.ntile = (B + scaml::kGradCT - 1) / scaml::kGradCT;
+  g.nsplit = scaml::grad_nsplit(M, g.ntile, num_sms());
+  g.part = ws;
+  g.aal = g.part + (size_t)g.nsplit * (size_t)B * 2 * (size_t)d;
+  g.kernel_t = kernel_t;
+  scaml::QBlockVjpParams p{};
+  p.n_valid = n_valid, p.X = X, p.theta = theta, p.ystd = ystd, p.w = w, p.Xc = Xc, p.gcov = g_cov, p.gmean = g_mean;
+  p.U = U, p.beta = beta, p.beta_f = beta_f, p.theta_t = theta_t, p.dmean = dmean, p.dvar = dvar, p.dX = dX;
+  p.s2t = g.s_all * g.s_all;
+  p.M = M, p.n_max = n_max, p.n_pad = g.n_pad, p.d = d, p.B = B, p.B_p = g.B_p, p.q = q, p.n_t = n_t, p.n_tp = n_tp;
+  p.kernel_t = kernel_t;
+  return scaml::launch_qblock_vjp(p, g, kernel, num_sms(), stream);
 }
 
 #endif

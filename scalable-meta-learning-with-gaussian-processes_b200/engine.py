@@ -613,6 +613,49 @@ class Engine:
         self.launches += 2
         return dmean, dvar
 
+    # ---- joint q-point blocks (batch acquisition: autograd through ScaMLGP.forward with q > 1) ---------------- #
+    def _grad_ws(self, need: int) -> torch.Tensor:
+        if self._gws is None or self._gws.numel() * 8 < need:
+            self._gws = torch.empty((need + 7) // 8, dtype=torch.float64, device=self.device)
+        return self._gws
+
+    def qblock_cov(self, fs: FittedSources, w: torch.Tensor, Xc: torch.Tensor, U: torch.Tensor, q: int) -> torch.Tensor:
+        """Weighted prior block [B / q, q, q] of every block of q consecutive points of Xc [B, d] (raw-Y units), from
+        U = cond_prepare(fs, Xc, w); U is left unchanged.  B <= 128, q <= 16."""
+        b = fs.batch
+        B, d = Xc.shape
+        w = w.to(torch.float64).contiguous()
+        cov = torch.empty(B // q, q, q, dtype=torch.float64, device=self.device)
+        need = self.lib.qblock_cov_workspace_bytes(b.M, B, q)
+        ws = self._grad_ws(need)
+        self.lib.qblock_cov(_ptr(b.X), _ptr(b.n_valid), _ptr(fs.theta), _ptr(b.ystd), _ptr(w), _ptr(Xc), _ptr(U), _ptr(cov),
+                            _ptr(ws), need, b.M, b.n_max, d, B, q, fs.spec.kernel, self._stream())
+        self.launches += 2
+        return cov
+
+    def qblock_vjp(self, fs: FittedSources, w: torch.Tensor, Xc: torch.Tensor, U: torch.Tensor, q: int,
+                   g_mean: torch.Tensor, g_cov: torch.Tensor, theta_t: torch.Tensor, kernel_t: int,
+                   ts: Optional["TargetState"] = None, A: Optional[torch.Tensor] = None,
+                   beta: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """dX [B, d] = d a / d Xc for the upstream gradients g_mean [B] = d a / d mean and g_cov [B / q, q, q] =
+        d a / d Sigma of the joint block posterior (un-standardised).  Inputs as for `posterior_grad`, plus the
+        constrained target-kernel parameters theta_t [P] (its kernel enters every block).  U is consumed."""
+        b = fs.batch
+        B, d = Xc.shape
+        n_t = 0 if ts is None else ts.Xt.shape[0]
+        w = w.to(torch.float64).contiguous()
+        g_mean = g_mean.to(self.device, torch.float64).contiguous()
+        g_cov = g_cov.to(self.device, torch.float64).contiguous()
+        dX = torch.empty(B, d, dtype=torch.float64, device=self.device)
+        need = self.lib.qblock_vjp_workspace_bytes(b.M, b.n_max, d, B, n_t)
+        ws = self._grad_ws(need)
+        self.lib.qblock_vjp(_ptr(b.X), _ptr(b.n_valid), _ptr(fs.theta), _ptr(fs.alpha), _ptr(b.ystd), _ptr(w), _ptr(Xc),
+                            _ptr(U), _ptr(ts.Xt) if n_t else None, _ptr(A), _ptr(ts.alpha) if n_t else None, _ptr(beta),
+                            _ptr(theta_t), ts.s_all if n_t else 1.0, _ptr(g_mean), _ptr(g_cov), _ptr(dX), _ptr(ws), need,
+                            b.M, b.n_max, d, B, q, n_t, fs.spec.kernel, kernel_t, self._stream())
+        self.launches += 6 if n_t else 4  # fold (+ beta fold, mix), contract, finish, direct terms
+        return dX
+
 
 @dataclass
 class TargetState:

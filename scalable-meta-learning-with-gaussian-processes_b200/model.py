@@ -598,6 +598,81 @@ class ScaMLGP:
             outs.append((mean, var, dm, dv))
         return tuple(torch.cat([o[i] for o in outs]).to(X.device) for i in range(4))
 
+    def posterior_blocks(self, X: torch.Tensor):
+        """Joint posterior of b blocks of q points, X [b, q, d], 1 <= q <= 16, and its vector-Jacobian product.
+
+        Returns mean [b, q], cov [b, q, q] (un-standardised, the blocks `posterior(X)` returns for q > 1) and
+        `vjp(g_mean [b, q], g_cov [b, q, q]) -> dX [b, q, d]`, the gradient wrt X of sum(g_mean mean) + sum(g_cov cov):
+        what a batch acquisition (qUCB, qEI) hands back from autograd on the small (mean, cov) leaves.  The blocks
+        come from U = K_m^-1 k*_m on the tensor cores (`cond_prepare` at the points) and `csrc/scaml_qblock.cuh`,
+        in launches of <= 128 points that never split a block.  `vjp` may be called once: it consumes the U of every
+        launch, which stay allocated until then (one [M, n_pad, 128] array per 128 points)."""
+        eng, dev = self.engine, self.engine.device
+        if X.dim() != 3:
+            raise ValueError(f"posterior_blocks expects X [b, q, d], got shape {tuple(X.shape)}")
+        nb_all, q, d = X.shape
+        if self._sharded is not None:
+            raise NotImplementedError("q-point blocks are not available for task-sharded source GPs (group=)")
+        if not 1 <= q <= 16:
+            raise NotImplementedError(f"q-point blocks cover 1 <= q <= 16 points per block, got q = {q}")
+        if not self.supports_candidate_gradients:
+            raise NotImplementedError("q-point blocks need n <= 512 points per task, d <= 16 and n_t <= 128")
+        fs, n_t = self._fitted, self.num_train
+        Xall = X.reshape(-1, d).to(dev, DT).contiguous()
+        w = self.pruned_weights()
+        kernel_t = self.hyper_spec().kernel
+        if n_t > 0:
+            ts = self._target_state()
+            theta_t = ts.theta.clone()
+            theta_t[d + 1] = 0.0  # noise-free kernel values
+            if self._condA is None:
+                self._condA = eng.cond_prepare(fs, self._Xt)
+        else:
+            ts, theta_t = None, self._target_kernel_theta(d).reshape(-1)
+        step = (128 // q) * q
+        idx = torch.arange(step, device=dev).reshape(-1, q)
+        means, covs, launches = [], [], []
+        for lo in range(0, Xall.shape[0], step):
+            Xc = Xall[lo:lo + step].contiguous()
+            nb = Xc.shape[0] // q
+            U = eng.cond_prepare(fs, Xc, w)  # pruned tasks skipped
+            cov = eng.qblock_cov(fs, w, Xc, U, q)
+            Z = torch.cat([self._Xt, Xc]) if n_t > 0 else Xc
+            kt = eng.kernel_matrix(Z.unsqueeze(0).contiguous(), theta_t.reshape(1, -1), kernel_t)[0]
+            ib = idx[:nb]
+            kqq = kt[n_t:, n_t:][ib.unsqueeze(2), ib.unsqueeze(1)]  # [nb, q, q] diagonal blocks
+            beta = None
+            if n_t > 0:
+                pm, pv, cross = eng.prior_values(fs, w, Xc, U, self._Xt, self._condA)
+                mean, _, beta = eng.target_posterior_beta(ts, pm, pv, cross, Xc)
+                S2 = ts.s_all ** 2
+                ks = (cross / S2 + kt[n_t:, :n_t]).reshape(nb, q, n_t)  # standardised cross-covariance with X_t
+                cov = cov + S2 * (kqq - ks @ beta[:, :n_t].reshape(nb, q, n_t).transpose(1, 2))
+                cov = 0.5 * (cov + cov.transpose(1, 2))
+            else:  # prior-only model (optimizer.py:135-141): no outcome transform
+                mean = eng.values_from_u(fs, w, Xc, U)[0]
+                cov = cov + kqq
+            means.append(mean.reshape(nb, q))
+            covs.append(cov)
+            launches.append((lo, Xc, U, beta))
+        consumed = []
+
+        def vjp(g_mean: torch.Tensor, g_cov: torch.Tensor) -> torch.Tensor:
+            if consumed:
+                raise RuntimeError("the vjp of posterior_blocks can be called once (it consumes the cached U)")
+            consumed.append(True)
+            gm = g_mean.reshape(-1).to(dev, DT)
+            gc = g_cov.reshape(-1, q, q).to(dev, DT)
+            outs = []
+            for lo, Xc, U, beta in launches:
+                B = Xc.shape[0]
+                outs.append(eng.qblock_vjp(fs, w, Xc, U, q, gm[lo:lo + B], gc[lo // q:(lo + B) // q], theta_t, kernel_t,
+                                           ts, self._condA if n_t > 0 else None, beta))
+            launches.clear()
+            return torch.cat(outs).reshape(nb_all, q, d).to(X.device)
+
+        return torch.cat(means).to(X.device), torch.cat(covs).to(X.device), vjp
+
     def _posterior_fused(self, Xc: torch.Tensor, w: torch.Tensor):
         """n_t > 0, q = 1: prior mean / variance and the cross-covariance with the target inputs in ONE prediction
         launch (the k*^T A_m contraction rides on the k* tiles), then the n_t-dimensional conditioning."""

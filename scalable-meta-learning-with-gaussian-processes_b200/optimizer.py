@@ -21,7 +21,7 @@ import torch
 from .model import ScaMLGP, meta_fit_scamlgp
 from .space import (Evaluation, EvaluationsError, EvaluationSpecification, Objective, OptimizerNotReady,
                     ParameterSpace, filter_y_nans, impute_nans_with_constant, to_numerical)
-from .utils import UpperConfidenceBound, metadata_to_numerical, optimize_marginal_likelihood
+from .utils import UpperConfidenceBound, metadata_to_numerical, optimize_marginal_likelihood, qUpperConfidenceBound
 
 
 def optimize_acqf_batched(af: Callable[[torch.Tensor], torch.Tensor], bounds: np.ndarray, generator: torch.Generator,
@@ -51,16 +51,22 @@ def optimize_acqf_batched(af: Callable[[torch.Tensor], torch.Tensor], bounds: np
 
 
 def optimize_acqf_lbfgsb(af, bounds: np.ndarray, generator: torch.Generator, raw_samples: int = 1024,
-                         num_restarts: int = 32, maxiter: int = 60) -> torch.Tensor:
-    """Maximise af over the box `bounds` [d, 2] (q = 1) the way botorch's `optimize_acqf` does for the reference:
+                         num_restarts: int = 32, maxiter: int = 60, q: int = 1) -> torch.Tensor:
+    """Maximise af over the box `bounds` [d, 2] the way botorch's `optimize_acqf` does for the reference:
     raw-sample screening, then scipy L-BFGS-B on the SUM of the acquisition values of all restarts (they are
     independent, so one optimiser run drives them in lock-step; botorch gen_candidates_scipy) with the analytic
-    gradient of `af.value_and_grad` -- one posterior-with-gradient launch sequence per function evaluation."""
+    gradient of `af.value_and_grad` -- one posterior-with-gradient launch sequence per function evaluation.
+
+    q = 1: af takes candidates [B, d]; returns the best point [d].  q > 1: af is a batch acquisition over blocks
+    [b, q, d] (qUpperConfidenceBound, qExpectedImprovement); `raw_samples` random q-batches are screened and the
+    q points of every restart are optimised jointly (num_restarts x q x d variables); returns the best batch [q, d]."""
     from scipy.optimize import minimize
 
     lo = torch.tensor(bounds[:, 0], dtype=torch.float64)
     hi = torch.tensor(bounds[:, 1], dtype=torch.float64)
     d = lo.numel()
+    if q > 1:
+        return optimize_acqf_lbfgsb_blocks(af, bounds, generator, raw_samples, num_restarts, maxiter, q)
     X0 = lo + (hi - lo) * torch.rand(raw_samples, d, dtype=torch.float64, generator=generator)
     v0 = af(X0).reshape(-1).cpu()
     top = torch.topk(v0, min(num_restarts, raw_samples))
@@ -77,6 +83,34 @@ def optimize_acqf_lbfgsb(af, bounds: np.ndarray, generator: torch.Generator, raw
                    options=dict(maxiter=int(maxiter)))
     Xo = torch.minimum(torch.maximum(torch.from_numpy(res.x.reshape(S, d).copy()), lo), hi)
     # never worse than the best raw sample: score the refined points and the starts together
+    cand = torch.cat([Xo, starts])
+    vals = af(cand).reshape(-1).cpu()
+    return cand[int(torch.argmax(vals))]
+
+
+def optimize_acqf_lbfgsb_blocks(af, bounds: np.ndarray, generator: torch.Generator, raw_samples: int = 1024,
+                                num_restarts: int = 32, maxiter: int = 60, q: int = 1) -> torch.Tensor:
+    """`optimize_acqf_lbfgsb` for a batch acquisition over blocks [b, q, d], any q >= 1; returns the best batch [q, d]."""
+    from scipy.optimize import minimize
+
+    lo = torch.tensor(bounds[:, 0], dtype=torch.float64)
+    hi = torch.tensor(bounds[:, 1], dtype=torch.float64)
+    d = lo.numel()
+    X0 = lo + (hi - lo) * torch.rand(raw_samples, q, d, dtype=torch.float64, generator=generator)
+    v0 = af(X0).reshape(-1).cpu()
+    top = torch.topk(v0, min(num_restarts, raw_samples))
+    starts = X0[top.indices].clone()
+    S = starts.shape[0]
+
+    def fun(xflat: np.ndarray):
+        X = torch.from_numpy(xflat.reshape(S, q, d).copy())
+        val, grad = af.value_and_grad(X)
+        return -float(val.sum()), -grad.cpu().numpy().reshape(-1).astype(np.float64)
+
+    res = minimize(fun, starts.numpy().reshape(-1), jac=True, method="L-BFGS-B",
+                   bounds=[(float(lo[k]), float(hi[k])) for _ in range(S * q) for k in range(d)],
+                   options=dict(maxiter=int(maxiter)))
+    Xo = torch.minimum(torch.maximum(torch.from_numpy(res.x.reshape(S, q, d).copy()), lo), hi)
     cand = torch.cat([Xo, starts])
     vals = af(cand).reshape(-1).cpu()
     return cand[int(torch.argmax(vals))]
@@ -200,15 +234,20 @@ class ScaMLGPBO(_SingleObjectiveBase):
                  max_pending_evaluations: Optional[int] = 1, num_restarts_log_likelihood: int = 5,
                  model_kwargs: Optional[Dict[str, Any]] = None, logger: Optional[logging.Logger] = None,
                  seed: Optional[int] = None, torch_dtype: torch.dtype = torch.float64, *, engine=None,
-                 fit_options: Optional[dict] = None, group=None):
+                 fit_options: Optional[dict] = None, group=None,
+                 batch_acquisition_function_factory: Optional[Callable] = None):
         """Single objective meta-learning BO optimizer with ScaML-GP as surrogate
         (reference scamlgp/optimizer.py:28-154: same arguments; `engine` / `fit_options` / `group` are additions).
 
         group: torch.distributed process group (True = default group): the meta-tasks are block-partitioned over its
         ranks -- the meta-fit (optimizer.py:128-133), the per-report caches (model.py:278-289) and every posterior
         (model.py:364-375) fan out over the GPUs with one all_gather / all_reduce each (sharded.py).  Every rank
-        runs the same optimizer with the same seed and proposes the same configurations."""
+        runs the same optimizer with the same seed and proposes the same configurations.
+
+        batch_acquisition_function_factory: model -> batch acquisition over q-point blocks, used by
+        `generate_evaluation_specifications(q)`; default qUpperConfidenceBound (beta = 9)."""
         n_features = len(search_space)
+        self.batch_acquisition_function_factory = batch_acquisition_function_factory or qUpperConfidenceBound
         batch_shape = torch.Size()
         if acquisition_function_factory is None:
             acquisition_function_factory = UpperConfidenceBound
@@ -228,6 +267,36 @@ class ScaMLGPBO(_SingleObjectiveBase):
                          num_initial_random_samples=num_initial_random_samples,
                          max_pending_evaluations=max_pending_evaluations, batch_shape=batch_shape, logger=logger,
                          seed=seed, torch_dtype=torch_dtype)
+
+    def generate_evaluation_specifications(self, q: int) -> List[EvaluationSpecification]:
+        """q configurations chosen jointly, for q concurrent workers; all are registered as pending.
+
+        The batch acquisition (`batch_acquisition_function_factory`) sees the model conditioned on the evaluations
+        already pending (the kriging-believer fantasy of `generate_evaluation_specification`) and L-BFGS-B optimises
+        the q points together.  Before `num_initial_random_samples` observations exist the q points are random
+        samples.  Raises OptimizerNotReady when pending + q exceeds `max_pending_evaluations`, NotImplementedError
+        for search spaces that are not all continuous and for q > 16."""
+        q = int(q)
+        if q < 1:
+            raise ValueError(f"q must be at least 1, got {q}")
+        if not self.search_space.is_all_continuous:
+            raise NotImplementedError("batch proposals (q points at once) cover all-continuous search spaces")
+        if (self.max_pending_evaluations is not None
+                and len(self.pending_specifications) + q > self.max_pending_evaluations):
+            raise OptimizerNotReady(f"{len(self.pending_specifications)} evaluations are pending, {q} more requested "
+                                    f"(max_pending_evaluations = {self.max_pending_evaluations})")
+        n_valid = int((~torch.isnan(self.losses)).sum())
+        if len(self.X) < self.num_initial_random or (self.num_initial_random > 0 and n_valid == 0):
+            return [self._spec(self.search_space.sample()) for _ in range(q)]
+        af = self.batch_acquisition_function_factory(self._model_for_acquisition())
+        if getattr(af, "maximize", False):
+            raise ValueError("Only acquisition functions to be minimized are supported")
+        kw = self.af_opt_kwargs
+        X = optimize_acqf_lbfgsb_blocks(af, self.search_space.numerical_bounds(), self._gen,
+                                        raw_samples=int(kw.get("raw_samples", 1024)),
+                                        num_restarts=int(kw.get("num_restarts", 32)),
+                                        maxiter=int(kw.get("maxiter", 60)), q=q)
+        return [self._spec(self.search_space.from_numerical(x.numpy())) for x in X.reshape(q, -1)]
 
     def report(self, evaluations: Union[Evaluation, Iterable[Evaluation]]):
         """Book-keep the evaluations and refit the ScaML-GP target model (reference optimizer.py:156-185)."""

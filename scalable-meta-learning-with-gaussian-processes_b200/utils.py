@@ -10,10 +10,12 @@ conversion/validation and the UCB acquisition, on the B200 engine.
   validate_meta_data             scamlgp/utils.py:112-136
   optimize_marginal_likelihood   scamlgp/utils.py:139-212
   UpperConfidenceBound           scamlgp/utils.py:215-224
+plus the batch (q > 1) acquisitions qUpperConfidenceBound / qExpectedImprovement (botorch's MC semantics).
 """
 from __future__ import annotations
 
 import logging
+import math
 import warnings
 from typing import Dict, Hashable, Iterable, Optional, Union
 
@@ -192,3 +194,115 @@ class UpperConfidenceBound:
         sig = torch.sqrt(self.beta * var.clamp_min(1e-9))
         grad = -dmean + (0.5 * self.beta / sig * live.to(sig.dtype)).unsqueeze(-1) * dvar
         return -mean + sig, grad
+
+
+def psd_safe_cholesky(A: torch.Tensor) -> torch.Tensor:
+    """Cholesky factor of a batch of matrices [..., q, q] with linear_operator's psd_safe_cholesky jitter ladder: a
+    matrix whose factorisation fails is retried with 1e-8, 1e-7, 1e-6 added to its diagonal (differentiable)."""
+    from ._capi import NotPSDError
+    from .engine import JITTER_LADDER
+
+    L, info = torch.linalg.cholesky_ex(A)
+    if not bool((info > 0).any()):
+        return L
+    eye = torch.eye(A.shape[-1], dtype=A.dtype, device=A.device)
+    for jit in JITTER_LADDER:
+        bad = (info > 0).to(A.dtype)[..., None, None]
+        L, info = torch.linalg.cholesky_ex(A + bad * jit * eye)
+        if not bool((info > 0).any()):
+            return L
+    raise NotPSDError(f"Matrix not positive definite after repeatedly adding jitter up to {JITTER_LADDER[-1]:.1e}")
+
+
+def sobol_normal_samples(num_samples: int, q: int, seed: int) -> torch.Tensor:
+    """[num_samples, q] scrambled-Sobol standard normal draws (botorch's draw_sobol_normal_samples: inverse CDF of
+    the Sobol points pulled in by one ulp so that no draw is infinite)."""
+    u = torch.quasirandom.SobolEngine(dimension=q, scramble=True, seed=seed).draw(num_samples, dtype=DT)
+    u = 0.5 + (1.0 - torch.finfo(DT).eps) * (u - 0.5)
+    return torch.erfinv(2.0 * u - 1.0) * math.sqrt(2.0)
+
+
+class _MCBatchAcquisition:
+    """Monte-Carlo acquisition over blocks of q points X [b, q, d] (botorch's MCAcquisitionFunction with a
+    SobolQMCNormalSampler): samples xi = mu + L z of the joint posterior of every block, L its Cholesky factor, z a
+    fixed scrambled-Sobol draw taken once per object (and q) so that an optimiser sees a deterministic function.
+    Values and gradients come from `ScaMLGP.posterior_blocks`; the gradient is autograd on the small (mu, Sigma)
+    leaves followed by the model's vector-Jacobian product (csrc/scaml_qblock.cuh)."""
+
+    maximize = False
+
+    def __init__(self, model, num_samples: int = 128, seed: int = 0):
+        self.model = model
+        self.num_samples = int(num_samples)
+        self.seed = int(seed)
+        self._z: Dict[int, torch.Tensor] = {}
+
+    def base_samples(self, q: int) -> torch.Tensor:
+        if q not in self._z:
+            self._z[q] = sobol_normal_samples(self.num_samples, q, self.seed)
+        return self._z[q]
+
+    def from_moments(self, mean: torch.Tensor, cov: torch.Tensor) -> torch.Tensor:
+        """Acquisition value [b] of blocks with posterior mean [b, q] and covariance [b, q, q] (differentiable)."""
+        z = self.base_samples(mean.shape[-1]).to(mean.device)
+        L = psd_safe_cholesky(cov)
+        samples = mean.unsqueeze(-2) + torch.einsum("bik,sk->bsi", L, z)  # [b, num_samples, q]
+        return self._reduce(mean, samples)
+
+    def _reduce(self, mean: torch.Tensor, samples: torch.Tensor) -> torch.Tensor:
+        raise NotImplementedError
+
+    def __call__(self, X: torch.Tensor) -> torch.Tensor:
+        return self.forward(X)
+
+    def forward(self, X: torch.Tensor) -> torch.Tensor:
+        """Values [b] of the blocks X [b, q, d]; evaluated 128 points at a time (each launch's U is freed before the
+        next one is built)."""
+        step = max(1, 128 // X.shape[-2])
+        vals = []
+        for lo in range(0, X.shape[0], step):
+            mean, cov, _ = self.model.posterior_blocks(X[lo:lo + step])
+            vals.append(self.from_moments(mean, cov))
+        return torch.cat(vals)
+
+    def value_and_grad(self, X: torch.Tensor):
+        """Values [b] and their gradients wrt the blocks [b, q, d]."""
+        mean, cov, vjp = self.model.posterior_blocks(X)
+        m, c = mean.detach().requires_grad_(True), cov.detach().requires_grad_(True)
+        with torch.enable_grad():
+            val = self.from_moments(m, c)
+            g_mean, g_cov = torch.autograd.grad(val.sum(), (m, c))
+        return val.detach(), vjp(g_mean, g_cov)
+
+
+class qUpperConfidenceBound(_MCBatchAcquisition):
+    """botorch's qUpperConfidenceBound turned into minimisation like `UpperConfidenceBound`:
+    mean over the samples of max_i ( -mu_i + sqrt(beta pi / 2) |xi_i - mu_i| ).  At q = 1 its expectation is the
+    analytic -mu + sqrt(beta sigma^2)."""
+
+    def __init__(self, model, beta: Union[float, torch.Tensor] = 9.0, num_samples: int = 128, seed: int = 0):
+        super().__init__(model, num_samples, seed)
+        self.beta = float(beta)
+
+    def _reduce(self, mean, samples):
+        scale = math.sqrt(self.beta * math.pi / 2.0)
+        return (-mean.unsqueeze(-2) + scale * (samples - mean.unsqueeze(-2)).abs()).max(dim=-1).values.mean(dim=-1)
+
+
+class qExpectedImprovement(_MCBatchAcquisition):
+    """botorch's qExpectedImprovement for a loss to be minimised: mean over the samples of max_i max(best_f - xi_i, 0).
+    best_f defaults to the smallest observed loss of the model's training data."""
+
+    def __init__(self, model, best_f: Optional[Union[float, torch.Tensor]] = None, num_samples: int = 128,
+                 seed: int = 0):
+        super().__init__(model, num_samples, seed)
+        if best_f is None:
+            Y = model._train_Y.reshape(-1)
+            Y = Y[~torch.isnan(Y)]
+            if Y.numel() == 0:
+                raise ValueError("qExpectedImprovement needs best_f when the model has no observations")
+            best_f = Y.min()
+        self.best_f = float(best_f)
+
+    def _reduce(self, mean, samples):
+        return (self.best_f - samples).clamp_min(0.0).max(dim=-1).values.mean(dim=-1)
