@@ -126,6 +126,11 @@ int scaml_factorize_ladder(const double* X, const double* y, const int32_t* n_va
                            int M, int n_max, int d, const scaml_hyper_spec* spec, void* stream);
 
 
+/* Largest n_max the prediction kernel (scaml_predict_weighted, scaml_predict_conditioned) accepts at input
+ * dimension d: its k* tiles, the L^-1 ring and the staged inputs must fit 227 KB (576 for d <= 6, 512 at
+ * d = 10, 320 at d = 16, 256 at d = 32); 0 for d outside 1..32. */
+int scaml_predict_max_points(int d);
+
 /* Bytes of partial-sum scratch scaml_predict_weighted needs for B candidates. */
 size_t scaml_predict_workspace_bytes(int M, int n_max, int d, int B);
 
@@ -150,7 +155,9 @@ int scaml_predict_weighted(const double* X, const int32_t* n_valid, const double
  * reduce = 1: mean [nA] = sum_m w_m mean_m, cov [nA][nB] = sum_m w_m^2 Sigma_m in a fixed order --
  *             the joint prior blocks `ScaMLGP.forward` builds in eval mode
  *             (reference scamlgp/model.py:364-375 via _compute_target_prior :108-135).
- * n_max <= 256 in this release (k(X,A), k(X,B) are held in shared memory). */
+ * n_max <= scaml_predict_cross_max_points(d) (k(X,A), k(X,B) are held in shared memory: 256 for d <= 24,
+ * 192 above). */
+int scaml_predict_cross_max_points(int d);
 size_t scaml_predict_cross_workspace_bytes(int M, int nA, int nB, int reduce);
 int scaml_predict_cross(const double* X, const int32_t* n_valid, const double* theta,
                         const double* linv_packed, const double* alpha, const double* ybar,

@@ -100,8 +100,10 @@ EXPORTED_SYMBOLS = (
     "scaml_lml_grad_ladder",
     "scaml_factorize",
     "scaml_factorize_ladder",
+    "scaml_predict_max_points",
     "scaml_predict_workspace_bytes",
     "scaml_predict_weighted",
+    "scaml_predict_cross_max_points",
     "scaml_predict_cross_workspace_bytes",
     "scaml_predict_cross",
     "scaml_target_workspace_bytes",
@@ -205,6 +207,10 @@ class ScamlLib:
         L.scaml_target_workspace_bytes.argtypes = [i32, i32]
         L.scaml_target_max_points.argtypes = [i32]
         L.scaml_target_max_points.restype = i32
+        L.scaml_predict_max_points.argtypes = [i32]
+        L.scaml_predict_max_points.restype = i32
+        L.scaml_predict_cross_max_points.argtypes = [i32]
+        L.scaml_predict_cross_max_points.restype = i32
         L.scaml_target_lml_grad_ladder.argtypes = ([vp] * 6 + [C.c_double, C.c_double] + [vp] * 5 +
                                                    [sz, i32, i32, i32, i32, C.POINTER(CHyperSpec), i32, C.c_double,
                                                     C.c_double, vp])
@@ -356,6 +362,12 @@ class ScamlLib:
 
     def target_max_points(self, d: int) -> int:
         return int(self.lib.scaml_target_max_points(int(d)))
+
+    def predict_max_points(self, d: int) -> int:
+        return int(self.lib.scaml_predict_max_points(int(d)))
+
+    def predict_cross_max_points(self, d: int) -> int:
+        return int(self.lib.scaml_predict_cross_max_points(int(d)))
 
     def target_lml_grad(self, smeans, scovs, Xt, yt, w, theta_raw, jitter, mu_all, s_all, lml, grad_w, grad_theta,
                         info, ws, ws_bytes, M, n_t, d, R, spec: HyperSpec, w_prior=(PRIOR_GAMMA, 1.0, 1.0), stream=0):

@@ -11,6 +11,8 @@
 // could expose between barriers are NOT detected (compute-sanitizer on the GPU box is
 // used for that).
 #pragma once
+#include <cxxabi.h>
+#include <dlfcn.h>
 #include <pthread.h>
 #include <sched.h>
 
@@ -19,6 +21,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <string>
 #include <thread>
 #include <vector>
 
@@ -104,8 +107,28 @@ inline void dmma884(double (&d)[2], double a, double b) {
   warp_sync();
 }
 
+// launch log: the demangled name of every kernel launched (e.g. "void scaml::scaml_grad_contract_kernel<0, 32>(...)"),
+// so tests can check which template instantiation a shape dispatches to
+inline std::vector<std::string>& launch_log() {
+  static std::vector<std::string> v;
+  return v;
+}
+template <class F>
+void log_launch(F kernel) {
+  Dl_info info;
+  std::string name = "?";
+  if (dladdr(reinterpret_cast<void*>(kernel), &info) != 0 && info.dli_sname != nullptr) {
+    int status = 0;
+    char* dem = abi::__cxa_demangle(info.dli_sname, nullptr, nullptr, &status);
+    name = (status == 0 && dem != nullptr) ? dem : info.dli_sname;
+    std::free(dem);
+  }
+  launch_log().push_back(name);
+}
+
 template <class F, class... A>
 void launch(dim3 grid, dim3 block, size_t smem_bytes, F kernel, A... args) {
+  log_launch(kernel);
   gDim() = grid;
   bDim() = block;
   const int nt = (int)block.x;

@@ -138,6 +138,7 @@ namespace {
 __attribute__((visibility("hidden"))) int scaml_detail_dispatch_fit8(const scaml::FitParams& p, int grid, size_t smem,
                                                                    void* stream);
 namespace {
+bool fit8_by_default(int n_pad) { return n_pad > 512; }
 bool use_fit8(int n_pad, int kernel) {
   if (const char* env = getenv("SCAML_FIT_IMPL")) {
     const int v = atoi(env);
@@ -145,7 +146,11 @@ bool use_fit8(int n_pad, int kernel) {
     if (v == 8) return true;
   }
   (void)kernel;
-  return n_pad > 512;
+  return fit8_by_default(n_pad);
+}
+// shared memory of the fit kernel the default dispatch picks at n_pad
+size_t fit_default_smem_bytes(int n_pad, int d) {
+  return fit8_by_default(n_pad) ? scaml::f8::smem_bytes(n_pad, d) : scaml::fit_smem_bytes(n_pad, d);
 }
 
 int dispatch_fit(const scaml::FitParams& p, int grid, size_t smem, void* stream) {
@@ -221,6 +226,19 @@ extern "C" {
 void scaml_debug_exp_nonpos(const double* x, double* out, int n) {
   for (int i = 0; i < n; ++i) out[i] = scaml::exp_nonpos(x[i]);
 }
+// tests only: the kernels launched since the last clear, one demangled name per line; returns the length of the
+// whole text (written up to cap - 1 characters and NUL-terminated when cap > 0)
+size_t scaml_debug_launch_log(char* buf, size_t cap) {
+  std::string all;
+  for (const std::string& s : cuemu::launch_log()) all += s + "\n";
+  if (buf != nullptr && cap > 0) {
+    const size_t k = all.size() < cap - 1 ? all.size() : cap - 1;
+    std::memcpy(buf, all.data(), k);
+    buf[k] = '\0';
+  }
+  return all.size();
+}
+void scaml_debug_launch_log_clear(void) { cuemu::launch_log().clear(); }
 #endif
 #ifdef SCAML_ABLATE
 void scaml_debug_set_ablate(int bits) { cudaMemcpyToSymbol(scaml::g_ablate, &bits, sizeof(int)); }
@@ -241,8 +259,9 @@ const char* scaml_version(void) {
 int scaml_fit_limits(int* n_max_limit, int* d_limit) {
   if (d_limit) *d_limit = scaml::kMaxP - 2;
   if (n_max_limit) {
+    // the 8-warp kernel (n_pad > 512) stages 3 n_pad doubles, the 4-warp one 2 n_pad: the limit is the 8-warp one's
     int n = 64;
-    while (scaml::fit_smem_bytes(n + 64, 6) <= kMaxSmem) n += 64;
+    while (fit_default_smem_bytes(n + 64, 6) <= kMaxSmem) n += 64;
     *n_max_limit = n;
   }
   return 0;
@@ -317,6 +336,13 @@ int scaml_kernel_matrix(const double* X, const int32_t* n_valid, const double* t
   return scaml::launch_kmat(X, n_valid, theta, K, M, n_max, d, kernel, stream);
 }
 
+int scaml_predict_max_points(int d) {
+  if (d <= 0 || d > scaml::kMaxP - 2) return 0;
+  int n = 0, ct = 0, alias = 0;
+  while (scaml::predict_config(n + 64, d, &ct, &alias)) n += 64;
+  return n;
+}
+
 size_t scaml_predict_workspace_bytes(int M, int n_max, int d, int B) {
   return scaml::predict_workspace_bytes(M, pad64(n_max), d, B, num_sms());
 }
@@ -337,6 +363,13 @@ int scaml_predict_weighted(const double* X, const int32_t* n_valid, const double
 
 #endif
 #if SCAML_HAS(3)
+int scaml_predict_cross_max_points(int d) {
+  if (d <= 0 || d > scaml::kMaxP - 2) return 0;
+  int n = 0;
+  while (scaml::cross_smem_bytes(n + 64, d) <= (size_t)227 * 1024) n += 64;
+  return n;
+}
+
 size_t scaml_predict_cross_workspace_bytes(int M, int nA, int nB, int reduce) {
   return scaml::cross_workspace_bytes(M, nA, nB, reduce, num_sms());
 }

@@ -369,10 +369,19 @@ class Engine:
         return mean, cov
 
     # ---- conditioning at scale (cross-covariance fused into the prediction kernel) ------- #
+    def predict_supported(self, fs: FittedSources) -> bool:
+        """The prediction kernel (`predict_weighted`, `predict_conditioned`) accepts the tasks' (n_max, d)."""
+        return fs.batch.n_max <= self.lib.predict_max_points(fs.batch.d)
+
+    def cross_supported(self, fs: FittedSources) -> bool:
+        """The stand-alone cross-covariance kernel (`predict_cross`) accepts the tasks' (n_max, d)."""
+        return fs.batch.n_max <= self.lib.predict_cross_max_points(fs.batch.d)
+
     def cond_supported(self, fs: FittedSources, n_t: int) -> bool:
-        """The A_m-based conditioning kernels cover what the prediction kernel covers (n_max <= 512) and n_t <= 128."""
+        """The A_m-based conditioning kernels cover what the prediction kernel covers (n_max <= 512, and less for
+        d > 10: `predict_supported`), d <= 16 and n_t <= 128."""
         b = fs.batch
-        return 0 < n_t <= 128 and b.n_max <= 512 and b.d <= 16
+        return 0 < n_t <= 128 and b.n_max <= 512 and b.d <= 16 and self.predict_supported(fs)
 
     def cond_prepare(self, fs: FittedSources, Xt: torch.Tensor, w: Optional[torch.Tensor] = None) -> torch.Tensor:
         """A [M, n_pad, n_tp] with A_m = K_m^-1 K_m(X_m, X_t): once per set of target inputs.  With w given, tasks

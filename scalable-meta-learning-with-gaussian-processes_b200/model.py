@@ -305,6 +305,10 @@ class ScaMLGP:
             raise NotImplementedError(
                 f"{n_t} target observations with {self._fitted.batch.n_max} points per source task: the fused "
                 "conditioning kernels cover n_t <= 128 and the stand-alone cross-covariance kernel n <= 256")
+        if n_t > 0 and not (self.engine.cond_supported(self._fitted, n_t) or self.engine.cross_supported(self._fitted)):
+            raise NotImplementedError(f"{n_t} target observations with {self._limits_text()}: the source caches at "
+                                      "the target inputs need the fused conditioning kernels (n_t <= 128, d <= 16 and "
+                                      "the prediction kernel's n) or the cross-covariance kernel")
         self._Xt = train_X.reshape(n_t, d).to(dev, DT).contiguous()
         # cache the source posteriors at the target inputs (model.py:278-289): one launch for all tasks
         self._condA: Optional[torch.Tensor] = None  # K_m^-1 K_m(X_m, X_t) of every source task
@@ -381,6 +385,19 @@ class ScaMLGP:
         yield ("weights_prior", self, self.weights_prior, lambda m: m.weights, lambda m, v: m._set_weights(v))
 
     # ---- internals ---------------------------------------------------------------------------- #
+    def _limits_text(self) -> str:
+        b, lib = self._fitted.batch, self.engine.lib
+        return (f"{b.n_max} points per source task at d = {b.d} (the prediction kernel covers n <= "
+                f"{lib.predict_max_points(b.d)}, the cross-covariance kernel n <= {lib.predict_cross_max_points(b.d)})")
+
+    def _require_predict(self) -> None:
+        if not self.engine.predict_supported(self._fitted):
+            raise NotImplementedError(f"posterior with {self._limits_text()}: outside the prediction kernel")
+
+    def _require_cross(self, what: str) -> None:
+        if not self.engine.cross_supported(self._fitted):
+            raise NotImplementedError(f"{what} with {self._limits_text()}: outside the cross-covariance kernel")
+
     @property
     def num_train(self) -> int:
         return self._Xt.shape[0]
@@ -431,9 +448,17 @@ class ScaMLGP:
             mean = self.source_means @ w
             cov = self.source_covs @ w ** 2
         elif self._sharded is not None:
+            self._require_cross("joint prior (eval mode)")
             mean, cov = self._sharded.predict_cross(self.pruned_weights(), xd)
-        else:
+        elif eng.cross_supported(self._fitted):
             mean, cov = eng.predict_cross(self._fitted, xd, None, w=self.pruned_weights())
+        elif eng.cond_supported(self._fitted, xd.shape[0]):  # the points as their own "target inputs"
+            w = self.pruned_weights()
+            U = eng.cond_prepare(self._fitted, xd, w)
+            mean, _, cov = eng.predict_conditioned(self._fitted, w, xd, xd, U)
+            cov = 0.5 * (cov + cov.t())
+        else:
+            self._require_cross("joint prior (eval mode)")
         if self.outcome_transform is not None:
             mu, sd = float(self.outcome_transform.means), float(self.outcome_transform.stdvs)
             mean = (mean - mu) / sd
@@ -458,6 +483,7 @@ class ScaMLGP:
             X = X.reshape(-1, X.shape[-1])
         else:
             lead = None
+        self._require_predict()
         Xc = X.to(dev, DT).contiguous()
         w = self.pruned_weights()
         if self._sharded is not None:
@@ -533,6 +559,7 @@ class ScaMLGP:
         Sigma(Xf, X_t) [B, n_t] (None without target data), summed over ALL tasks."""
         eng, n_t = self.engine, self.num_train
         if self._sharded is not None:
+            self._require_cross("joint posterior")
             mean, cqq = self._sharded.predict_cross(w, Xf)
             cqt = self._sharded.predict_cross(w, Xf, self._Xt)[1] if n_t > 0 else None
             return mean, cqq, cqt
@@ -542,21 +569,24 @@ class ScaMLGP:
             mean, _, cqq = eng.predict_conditioned(fs, w, Xf, Xf, U)
             cqq = 0.5 * (cqq + cqq.t())
             cqt = None
-            if n_t > 0:
+            if n_t > 0 and eng.cond_supported(fs, n_t):
                 if self._condA is None:
                     self._condA = eng.cond_prepare(fs, self._Xt)
                 cqt = eng.predict_conditioned(fs, w, Xf, self._Xt, self._condA)[2]
+            elif n_t > 0:  # n_t > 128: the constructor made sure the cross-covariance kernel covers the tasks
+                cqt = eng.predict_cross(fs, Xf, self._Xt, w=w)[1]
             return mean, cqq, cqt
+        self._require_cross("joint posterior")
         mean, cqq = eng.predict_cross(fs, Xf, None, w=w)
         cqt = eng.predict_cross(fs, Xf, self._Xt, w=w)[1] if n_t > 0 else None
         return mean, cqq, cqt
 
     @property
     def supports_candidate_gradients(self) -> bool:
-        """Shapes the analytic-gradient kernels cover (n <= 512 points per task, d <= 16, n_t <= 128); outside them
-        the optimizer falls back to its zeroth-order acquisition search."""
+        """Shapes the analytic-gradient kernels cover (n <= 512 points per task and what the prediction kernel
+        covers, d <= 16, n_t <= 128); outside them the optimizer falls back to its zeroth-order acquisition search."""
         b = self._fitted.batch
-        return b.n_max <= 512 and b.d <= 16 and self.num_train <= 128
+        return b.n_max <= 512 and b.d <= 16 and self.num_train <= 128 and self.engine.predict_supported(self._fitted)
 
     def posterior_with_grad(self, X: torch.Tensor):
         """Posterior mean / variance [B] and their gradients wrt the candidates [B, d] (q = 1), un-standardised.
@@ -572,7 +602,9 @@ class ScaMLGP:
             X = X[:, 0, :]
         b = self._fitted.batch
         if not self.supports_candidate_gradients:
-            raise NotImplementedError("candidate gradients need n <= 512 points per task, d <= 16 and n_t <= 128")
+            raise NotImplementedError("candidate gradients need n <= 512 points per task (and within the prediction "
+                                      f"kernel), d <= 16 and n_t <= 128; the model has {self._limits_text()} and "
+                                      f"n_t = {self.num_train}")
         Xall = X.to(dev, DT).contiguous()
         w = self.pruned_weights()
         n_t = self.num_train
@@ -616,7 +648,9 @@ class ScaMLGP:
         if not 1 <= q <= 16:
             raise NotImplementedError(f"q-point blocks cover 1 <= q <= 16 points per block, got q = {q}")
         if not self.supports_candidate_gradients:
-            raise NotImplementedError("q-point blocks need n <= 512 points per task, d <= 16 and n_t <= 128")
+            raise NotImplementedError("q-point blocks need n <= 512 points per task (and within the prediction "
+                                      f"kernel), d <= 16 and n_t <= 128; the model has {self._limits_text()} and "
+                                      f"n_t = {self.num_train}")
         fs, n_t = self._fitted, self.num_train
         Xall = X.reshape(-1, d).to(dev, DT).contiguous()
         w = self.pruned_weights()

@@ -32,6 +32,12 @@ def _batch(pb):
     (2, 1, 512, 10, None, 0),           # config 4 shape, sampled
     (3, 2, 128, 17, [128, 90, 3], 0),   # d > 8: input dimensions beyond the register-prefetched ones
     (2, 1, 320, 32, None, 3),           # d at the library limit, 5 super-tiles
+    (4, 1, 577, 6, [577, 400, 513, 10], 0),  # n_pad = 640 > 512: the default dispatch picks the 8-warp kernel;
+    (4, 1, 577, 6, [577, 400, 513, 10], 1),  # ragged n_valid on both sides of 512 in one batch
+    (4, 1, 577, 6, [577, 400, 513, 10], 2),
+    (4, 1, 577, 6, [577, 400, 513, 10], 3),
+    (2, 1, 1000, 4, [1000, 300], 0),
+    (3, 2, 100, 1, [100, 50, 3], 0),     # d = 1: the extreme of the input padding
 ])
 def test_lml_grad_matches_oracle(engine, M, R, n, d, nv, kernel):
     pb = make_problem(M, R, n, d, seed=3, n_valid=nv, kernel=kernel)
@@ -45,6 +51,12 @@ def test_lml_grad_matches_oracle(engine, M, R, n, d, nv, kernel):
     assert int(info.abs().max()) == 0
     assert lml_rel_err(lml.cpu().numpy(), v) < TOL_LML
     assert grad_rel_err(grad.cpu().numpy(), g) < TOL_GRAD
+    fs = engine.factorize(batch, pb["th"][:, 0].contiguous().cuda(), pb["cspec"])
+    assert int(fs.info.abs().max()) == 0
+    for m in range(M):
+        k = int(pb["nv"][m])
+        st = O.factorize(pb["X"][m, :k], pb["Y"][m, :k], pb["th"][m, 0], pb["ospec"])
+        assert rel_err(fs.alpha[m, :k].cpu().numpy(), st.alpha.numpy()) < 1e-8
 
 
 @pytest.mark.parametrize("impl", ["4", "8"])
@@ -151,6 +163,8 @@ def test_factorize_and_weighted_prediction(engine):
     (256, 20, 2, [256, 130, 64]),    # 64-candidate tiles, aliased staging (large d)
     (256, 6, 1, [256, 130, 64]),     # Matern-1/2: k* from direct differences (not smooth in r^2), no tensor-core distances
     (192, 7, 0, [192, 77, 3]),       # d = 7: the norm rows do not fit the contraction's padding (accumulator-init path)
+    (576, 1, 0, [576, 300, 2]),      # d = 1 at the prediction kernel's largest n (scaml_predict_max_points(1))
+    (256, 32, 3, [256, 200, 9]),     # d = 32: 32-candidate tiles at n_pad = 256
 ])
 def test_weighted_prediction_other_layouts(engine, n, d, kernel, nvs):
     M, B = len(nvs), 150
@@ -269,7 +283,18 @@ def test_predict_cross_per_task_and_reduced(engine, kernel, nA, nB):
 @pytest.mark.parametrize("kernel,nt,M", [(0, 40, 64), (3, 80, 33), (0, 116, 8), (2, 1, 5)])
 def test_target_lml_grad_matches_oracle(engine, kernel, nt, M):
     """a7: ScaMLGP.forward training branch + priors (reference model.py:319-338,359-383)."""
-    n, d, R = 64, 4, 3
+    _target_case(engine, kernel, nt, M, 4)
+
+
+@pytest.mark.parametrize("kernel,d", [(0, 2), (3, 16)])
+def test_target_lml_grad_above_shared_memory_limit(engine, kernel, d):
+    """The first n_t above scaml_target_max_points(d): the BIG variant of the target kernels."""
+    nt = engine.lib.target_max_points(d) + 1
+    _target_case(engine, kernel, nt, 5, d)
+
+
+def _target_case(engine, kernel, nt, M, d):
+    n, R = 64, 3
     pb = make_problem(M, 1, n, d, seed=17)
     batch = _batch(pb)
     fs = engine.factorize(batch, pb["th"][:, 0].contiguous().cuda(), pb["cspec"])

@@ -9,12 +9,12 @@ import torch
 
 from oracle import scaml_oracle as O
 from scamlgp_b200._capi import HyperSpec
-from tests.helpers import TOL_GRAD, make_problem, rel_err
+from tests.helpers import TOL_GRAD, TOL_MEAN_VAR, make_problem, rel_err
 
 DT = torch.float64
 
 
-def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3):
+def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3, coincide=False):
     from scamlgp_b200.engine import SourceBatch
 
     dev = eng.device
@@ -26,6 +26,10 @@ def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3):
               for m in range(M)]
     g = torch.Generator().manual_seed(seed + 100)
     Xc = torch.rand(B, d, dtype=DT, generator=g)
+    if coincide:  # candidates on source training inputs (r^2 = 0 against one row of K_m), and a repeated candidate
+        Xc[0] = pb["X"][0, 0]
+        Xc[1] = pb["X"][M - 1, int(pb["nv"][M - 1]) - 1]
+        Xc[B - 1] = Xc[0]
     w = torch.as_tensor(w, dtype=DT)
     otspec, ctspec = O.HyperSpec.target(kernel_t), HyperSpec.target(kernel_t)
     tht = O.initial_theta_raw(d, otspec) + 0.3 * torch.randn(d + 2, dtype=DT, generator=g)
@@ -35,9 +39,23 @@ def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3):
         if float(w[m]) == 0.0:
             assert float(U[m].abs().max()) == 0.0
     # ---- values from U (no second pass over the factors) == the prediction kernel ---------------------------------- #
+    # The two kernels round the sum over tasks and points of w_m ystd_m k*_mi alpha_mi differently.  They agree to 1e-11
+    # of the mean, or to a few ulps of the sum of the magnitudes of its terms where that is larger: for a nearly
+    # singular K_m (d = 1: 150 points on [0, 1], cond(K) ~ 1e7) the terms are ~1e5 times the mean they cancel to.
+    terms = sum(float(w[m]) * st.ystd * (O.kernel_matrix(Xc, st.X, st.ls, st.os, st.kernel).abs() @ st.alpha.abs())
+                for m, st in enumerate(states))
+    mean_floor = 5e-16 * float(terms.max())
+
+    def mean_agrees(a, ref):
+        return float((a - ref).abs().max()) < max(1e-11 * float(ref.abs().max()), mean_floor)
+
     pm0, pv0 = eng.predict_weighted(fs, wd, Xcd)
+    om0, ov0 = O.scaml_prior_predict(states, w, Xc)
+    assert rel_err(pm0.cpu().numpy(), om0.numpy()) < TOL_MEAN_VAR
+    prior_scale = sum(float(w[m]) ** 2 * float(st.os) * st.ystd ** 2 for m, st in enumerate(states))
+    assert float((pv0.cpu() - ov0).abs().max()) < TOL_MEAN_VAR * prior_scale  # variances: relative to the prior scale
     vm, vv, _ = eng.values_from_u(fs, wd, Xcd, U)
-    assert rel_err(vm.cpu().numpy(), pm0.cpu().numpy()) < 1e-11
+    assert mean_agrees(vm, pm0)
     assert float((vv - pv0).abs().max()) < 1e-10 * float(pv0.abs().max())
     # ---- prior only (n_t = 0): gradient of sum_m w_m mu_m and sum_m w_m^2 var_m ------------------------------------ #
     dm, dv = eng.posterior_grad(fs, wd, Xcd, U)
@@ -48,6 +66,8 @@ def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3):
         return e0
     # ---- conditioned on n_t target points ------------------------------------------------------------------------- #
     Xt = torch.rand(nt, d, dtype=DT, generator=g)
+    if coincide:  # a candidate on a target input
+        Xt[nt - 1] = Xc[2]
     Yt = torch.sin(3.0 * Xt).sum(1, keepdim=True) + 0.05 * torch.randn(nt, 1, dtype=DT, generator=g)
     cache = O.build_target_cache(states, Xt, Yt)
     Xtd = Xt.to(dev)
@@ -58,7 +78,7 @@ def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3):
     assert ts.info == 0
     pm, pv, cross = eng.predict_conditioned(fs, wd, Xcd, Xtd, A)
     vm, vv, vc = eng.values_from_u(fs, wd, Xcd, U, Xtd, A)
-    assert rel_err(vm.cpu().numpy(), pm.cpu().numpy()) < 1e-11
+    assert mean_agrees(vm, pm)
     assert float((vv - pv).abs().max()) < 1e-10 * float(pv.abs().max())
     assert float((vc - cross).abs().max()) < 1e-10 * float(cross.abs().max())
     mean0, var0 = eng.target_posterior(ts, pm, pv, cross, Xcd)
@@ -83,8 +103,11 @@ def _case(eng, M, n, d, B, nt, nvs, kernel, kernel_t, w, seed=3):
         vals.append(eng.target_posterior(ts, a, b_, c, Xq.contiguous()))
     fd_m = (vals[0][0] - vals[1][0]) / (2 * h)
     fd_v = (vals[0][1] - vals[1][1]) / (2 * h)
-    assert float((fd_m - dm[:, k]).abs().max()) < 1e-5 * max(1.0, float(dm.abs().max()))
-    assert float((fd_v - dv[:, k]).abs().max()) < 1e-5 * max(1.0, float(dv.abs().max()))
+    rows = torch.ones(B, dtype=torch.bool, device=dev)
+    if coincide and 1 in (kernel, kernel_t):  # Matern-1/2 has a kink at r = 0: no central difference there
+        rows[[0, 1, 2, B - 1]] = False
+    assert float((fd_m - dm[:, k])[rows].abs().max()) < 1e-5 * max(1.0, float(dm.abs().max()))
+    assert float((fd_v - dv[:, k])[rows].abs().max()) < 1e-5 * max(1.0, float(dv.abs().max()))
     return e0 + e1
 
 
@@ -100,9 +123,18 @@ def emu_engine(emu_lib):
     (3, 64, 2, 5, 4, None, 3, 2, [0.7, 0.0, 0.3]),            # Matern source / target kernels, a pruned task
     (2, 40, 9, 8, 3, None, 0, 0, [0.6, 0.4]),                 # d > 8 (16-wide register variant)
     (2, 33, 2, 3, 0, [33, 1], 1, 0, [1.0, 0.5]),              # prior only, single-point task, Matern-1/2
+    (2, 30, 17, 6, 5, None, 0, 0, [0.6, 0.4]),                # d > 16 (32-wide register variant)
+    (2, 24, 32, 4, 3, None, 3, 1, [0.6, 0.4]),                # d = 32, the library limit
+    (2, 30, 1, 5, 4, [30, 7], 2, 0, [0.6, 0.4]),              # d = 1
 ])
 def test_emu_posterior_grad_matches_oracle_autograd(emu_engine, M, n, d, B, nt, nvs, kernel, kernel_t, w):
     _case(emu_engine, M, n, d, B, nt, nvs, kernel, kernel_t, w)
+
+
+@pytest.mark.parametrize("kernel", [0, 1, 2, 3])
+def test_emu_posterior_grad_at_coincident_points(emu_engine, kernel):
+    """Candidates equal to a source training input, to a target input and to each other (r^2 = 0)."""
+    _case(emu_engine, 2, 30, 3, 6, 5, [30, 12], kernel, kernel, [0.6, 0.4], coincide=True)
 
 
 @pytest.mark.gpu
@@ -113,11 +145,28 @@ def test_emu_posterior_grad_matches_oracle_autograd(emu_engine, M, n, d, B, nt, 
     (3, 512, 4, 33, 20, [512, 300, 65], 2, 1, None),
     (3, 96, 16, 9, 5, None, 0, 0, None),
     (4, 64, 3, 16, 0, None, 0, 0, None),
+    (3, 96, 17, 20, 12, [96, 50, 9], 0, 0, None),   # d = 17 and 32: the DMAX = 32 instantiations, all source kernels
+    (3, 96, 17, 20, 12, None, 1, 0, None),
+    (3, 96, 17, 20, 12, None, 2, 2, None),
+    (3, 96, 17, 20, 12, None, 3, 3, None),
+    (3, 128, 32, 33, 70, [128, 64, 1], 0, 1, None),
+    (3, 128, 32, 33, 70, None, 1, 0, None),
+    (3, 128, 32, 33, 70, None, 2, 0, None),
+    (3, 128, 32, 33, 70, None, 3, 2, None),
+    (4, 200, 6, 64, 20, [200, 150, 64, 7], 1, 1, None),  # Matern-1/2 source
+    (3, 150, 1, 50, 30, [150, 40, 2], 0, 0, None),        # d = 1
 ])
 def test_gpu_posterior_grad_matches_oracle_autograd(engine, M, n, d, B, nt, nvs, kernel, kernel_t, w):
     if w is None:
         w = list(np.linspace(1.0, 2.0, M) / M)
     _case(engine, M, n, d, B, nt, nvs, kernel, kernel_t, w)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("kernel", [0, 1, 2, 3])
+def test_gpu_posterior_grad_at_coincident_points(engine, kernel):
+    """Candidates equal to a source training input, to a target input and to each other (r^2 = 0)."""
+    _case(engine, 3, 128, 6, 40, 12, [128, 60, 9], kernel, kernel, [0.5, 0.3, 0.2], coincide=True)
 
 
 @pytest.mark.gpu

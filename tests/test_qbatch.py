@@ -85,9 +85,14 @@ def _oracle_blocks(args, X):
     return torch.stack(ms), torch.stack(cs)
 
 
-def _blocks_case(eng, M, n, d, nb, q, nt, ragged, kernel, kernel_t, prune):
+def _blocks_case(eng, M, n, d, nb, q, nt, ragged, kernel, kernel_t, prune, coincide=False):
     model, args, g = _fitted_model(eng, M, n, d, nt, ragged, kernel, kernel_t, prune)
     X = torch.rand(nb, q, d, dtype=DT, generator=g)
+    if coincide:  # a repeated point inside a block, a point on a source training input and one on a target input
+        X[0, q - 1] = X[0, 0]
+        X[nb - 1, 0] = O.synthetic_tasks(M, n, d, seed=3)[0][0, 0]
+        if nt > 0:
+            X[nb - 1, q - 1] = model.train_inputs[0][0]
     mean, cov, vjp = model.posterior_blocks(X)
     assert mean.shape == (nb, q) and cov.shape == (nb, q, q)
     assert torch.equal(cov, cov.transpose(1, 2))
@@ -140,6 +145,8 @@ EMU_CASES = [
     (2, 24, 3, 43, 3, 4, False, 0, 1, False),   # 129 points: a 126-point launch and a partial one of 3
     (2, 24, 3, 7, 1, 4, False, 0, 0, False),    # q = 1 against the existing gradient path
     (2, 20, 2, 8, 16, 0, False, 0, 0, False),   # B q = 128: one full launch
+    (2, 260, 2, 2, 3, 3, False, 0, 0, False),   # n_pad = 320 > 256: the staged inputs of the cov kernel
+    (2, 24, 1, 3, 2, 3, False, 2, 0, False),    # d = 1
 ]
 
 
@@ -155,9 +162,43 @@ def test_emu_posterior_blocks_match_oracle(emu_engine, M, n, d, nb, q, nt, ragge
     (3, 256, 4, 11, 3, 128, False, 2, 1, False),  # n_t = 128
     (4, 64, 6, 45, 3, 0, False, 0, 0, False),     # prior only, partial last launch
     (4, 96, 6, 40, 1, 20, False, 0, 0, False),
+    (3, 320, 6, 8, 4, 12, True, 0, 0, False),   # n > 256
+    (3, 512, 4, 6, 3, 20, False, 2, 1, False),  # n = 512, the model's limit
+    (3, 150, 1, 10, 4, 9, False, 0, 0, False),  # d = 1
 ])
 def test_gpu_posterior_blocks_match_oracle(engine, M, n, d, nb, q, nt, ragged, kernel, kernel_t, prune):
     _blocks_case(engine, M, n, d, nb, q, nt, ragged, kernel, kernel_t, prune)
+
+
+def _blocks_beyond_model(eng, monkeypatch, d, kernel, nt):
+    """d = 17, 32: the engine's q-block kernels (DMAX = 32) run beyond the model's d <= 16; the model's own block
+    code is reused with its shape gate lifted, so the values and the VJP are checked against the oracle the same way."""
+    from scamlgp_b200.model import ScaMLGP
+
+    monkeypatch.setattr(ScaMLGP, "supports_candidate_gradients", property(lambda self: True))
+    _blocks_case(eng, 2, 24, d, 3, 3, nt, False, kernel, kernel, False)
+
+
+@pytest.mark.parametrize("d,kernel,nt", [(17, 0, 4), (32, 3, 0)])
+def test_emu_qblock_beyond_model_dimension(emu_engine, monkeypatch, d, kernel, nt):
+    _blocks_beyond_model(emu_engine, monkeypatch, d, kernel, nt)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("d,kernel,nt", [(17, 0, 10), (17, 1, 0), (32, 2, 10), (32, 3, 20)])
+def test_gpu_qblock_beyond_model_dimension(engine, monkeypatch, d, kernel, nt):
+    _blocks_beyond_model(engine, monkeypatch, d, kernel, nt)
+
+
+@pytest.mark.parametrize("kernel", [0, 1, 2, 3])
+def test_emu_posterior_blocks_at_coincident_points(emu_engine, kernel):
+    _blocks_case(emu_engine, 2, 24, 3, 3, 3, 4, False, kernel, kernel, False, coincide=True)
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("kernel", [0, 1, 2, 3])
+def test_gpu_posterior_blocks_at_coincident_points(engine, kernel):
+    _blocks_case(engine, 3, 128, 6, 8, 4, 12, False, kernel, kernel, False, coincide=True)
 
 
 @pytest.mark.gpu
@@ -222,6 +263,16 @@ def _acq_case(eng, nt):
         (rd,) = torch.autograd.grad(rv.sum(), Xg)
         assert rel_err(v.numpy(), rv.detach().numpy()) < 1e-7
         assert rel_err(dX.numpy(), rd.numpy()) < 1e-7
+    # coincident points (a repeated point in a block, a point on a target input): singular blocks go through the
+    # jitter ladder and the values and gradients stay finite
+    Xs = X.clone()
+    Xs[0, 1] = Xs[0, 0]
+    if nt > 0:
+        Xs[1, 2] = model.train_inputs[0][0]
+    for af in (qUpperConfidenceBound(model, beta=4.0, num_samples=64, seed=3),
+               qExpectedImprovement(model, best_f=None if nt > 0 else best_f, num_samples=64, seed=3)):
+        v, dX = af.value_and_grad(Xs)
+        assert bool(torch.isfinite(v).all()) and bool(torch.isfinite(dX).all())
     # q = 1: qUCB with 4096 samples is the analytic UCB up to the sampling error
     Xc = torch.rand(6, 1, 3, dtype=DT, generator=g)
     qv = qUpperConfidenceBound(model, beta=9.0, num_samples=4096)(Xc)
