@@ -133,7 +133,8 @@ void launch(dim3 grid, dim3 block, size_t smem_bytes, F kernel, A... args) {
   bDim() = block;
   const int nt = (int)block.x;
   const int nw = (nt + 31) / 32;
-  for (unsigned b = 0; b < grid.x; ++b) {
+  for (unsigned long long b = 0; b < (unsigned long long)grid.x * grid.y * grid.z; ++b) {
+    const dim3 cta((unsigned)(b % grid.x), (unsigned)(b / grid.x % grid.y), (unsigned)(b / grid.x / grid.y));
     BlockCtx c;
     c.nthreads = nt;
     pthread_barrier_init(&c.bar, nullptr, nt);
@@ -147,7 +148,7 @@ void launch(dim3 grid, dim3 block, size_t smem_bytes, F kernel, A... args) {
     std::memset(mem, 0xCD, smem_bytes + 1024);  // poison: uninitialised smem reads show up as NaN-ish
     c.dyn_smem = (unsigned char*)mem;
     ctx() = &c;
-    bIdx() = dim3(b, 0, 0);
+    bIdx() = cta;
     std::vector<std::thread> th;
     th.reserve(nt);
     for (int t = 0; t < nt; ++t)
@@ -159,8 +160,8 @@ void launch(dim3 grid, dim3 block, size_t smem_bytes, F kernel, A... args) {
     // canary: a kernel that writes past the dynamic shared memory it asked for would corrupt a neighbour on the GPU
     for (size_t i = smem_bytes; i < smem_bytes + 1024; ++i)
       if (((unsigned char*)mem)[i] != 0xCD) {
-        std::fprintf(stderr, "cuda_emu: CTA %u wrote past its %zu bytes of dynamic shared memory (offset %zu)\n", b,
-                     smem_bytes, i);
+        std::fprintf(stderr, "cuda_emu: CTA (%u, %u, %u) wrote past its %zu bytes of dynamic shared memory at %zu\n",
+                     cta.x, cta.y, cta.z, smem_bytes, i);
         std::abort();
       }
     pthread_barrier_destroy(&c.bar);

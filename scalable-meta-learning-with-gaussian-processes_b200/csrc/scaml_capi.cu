@@ -80,48 +80,14 @@ int fit_grid_slots(int n_pad, int d) {
   return num_sms() * c;
 }
 
-template <int KIND>
-int launch_fit(const scaml::FitParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(scaml::kFitThreads), smem, scaml::scaml_fit_kernel<KIND>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml::scaml_fit_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml::scaml_fit_kernel<KIND><<<grid, scaml::kFitThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-
 #endif
 #if SCAML_HAS(1)
-template <int KIND>
-int launch_fit8(const scaml::FitParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(scaml::f8::kThreads), smem, scaml::f8::scaml_fit8_kernel<KIND>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml::f8::scaml_fit8_kernel<KIND>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml::f8::scaml_fit8_kernel<KIND><<<grid, scaml::f8::kThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-
 }  // namespace
 __attribute__((visibility("hidden"))) int scaml_detail_dispatch_fit8(const scaml::FitParams& p, int grid, size_t smem,
                                                                    void* stream) {
-  switch (p.spec.kernel) {
-    case SCAML_KERNEL_RBF: return launch_fit8<SCAML_KERNEL_RBF>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN12: return launch_fit8<SCAML_KERNEL_MATERN12>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN32: return launch_fit8<SCAML_KERNEL_MATERN32>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN52: return launch_fit8<SCAML_KERNEL_MATERN52>(p, grid, smem, stream);
-    default: return SCAML_E_ARG;
-  }
+  return scaml::dispatch_kind(p.spec.kernel, [&](auto K) {
+    return scaml::launch(scaml::f8::scaml_fit8_kernel<K.value>, grid, scaml::f8::kThreads, smem, stream, p);
+  });
 }
 namespace {
 
@@ -154,13 +120,9 @@ size_t fit_default_smem_bytes(int n_pad, int d) {
 }
 
 int dispatch_fit(const scaml::FitParams& p, int grid, size_t smem, void* stream) {
-  switch (p.spec.kernel) {
-    case SCAML_KERNEL_RBF: return launch_fit<SCAML_KERNEL_RBF>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN12: return launch_fit<SCAML_KERNEL_MATERN12>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN32: return launch_fit<SCAML_KERNEL_MATERN32>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN52: return launch_fit<SCAML_KERNEL_MATERN52>(p, grid, smem, stream);
-    default: return SCAML_E_ARG;
-  }
+  return scaml::dispatch_kind(p.spec.kernel, [&](auto K) {
+    return scaml::launch(scaml::scaml_fit_kernel<K.value>, grid, scaml::kFitThreads, smem, stream, p);
+  });
 }
 
 size_t fit_tile_workspace_bytes(int n_max, int d) {
@@ -189,14 +151,9 @@ int run_fit(scaml::FitParams p, void* workspace, size_t workspace_bytes, void* s
   p.order = nullptr;
   if (p.skip != nullptr || p.n_valid != nullptr) {  // active rows, largest tasks first
     int32_t* order = p.sched + 2;
-#ifdef SCAML_EMU
-    cuemu::launch(dim3(1), dim3(scaml::kSchedThreads), 0, scaml::scaml_fit_schedule_kernel<0>, p.skip, p.n_valid, p.M, p.R,
-                  p.n_max, p.sched, order);
-#else
-    scaml::scaml_fit_schedule_kernel<0><<<1, scaml::kSchedThreads, 0, (cudaStream_t)stream>>>(p.skip, p.n_valid, p.M, p.R,
-                                                                                         p.n_max, p.sched, order);
-    if (cudaGetLastError() != cudaSuccess) return SCAML_E_ARG;
-#endif
+    if (scaml::launch(scaml::scaml_fit_schedule_kernel<0>, 1, scaml::kSchedThreads, 0, stream, p.skip, p.n_valid, p.M,
+                      p.R, p.n_max, p.sched, order) != 0)
+      return SCAML_E_ARG;
     p.order = order;
   } else {
 #ifdef SCAML_EMU

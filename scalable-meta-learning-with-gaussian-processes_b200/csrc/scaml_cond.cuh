@@ -427,56 +427,14 @@ __global__ void __launch_bounds__(256) scaml_cond_caches_kernel(const CondCaches
   }
 }
 
-template <int KIND>
-int launch_cond_caches_k(const CondCachesParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(256), smem, scaml_cond_caches_kernel<KIND>, p);
-  return 0;
-#else
-  cudaError_t err =
-      cudaFuncSetAttribute(scaml_cond_caches_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_cond_caches_kernel<KIND><<<grid, 256, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-
 inline int launch_cond_caches(CondCachesParams p, int kernel, int num_sms, void* stream) {
   p.n_tp = cond_ntp(p.n_t);
   const size_t smem = cond_caches_smem_bytes(p.d, p.n_t, p.n_tp);
   if (smem > 227 * 1024) return SCAML_E_SMEM;
-  int grid = p.M < 2 * num_sms ? p.M : 2 * num_sms;
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: return launch_cond_caches_k<SCAML_KERNEL_RBF>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN12: return launch_cond_caches_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN32: return launch_cond_caches_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream);
-    default: return launch_cond_caches_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream);
-  }
-}
-
-template <int KIND, int NJT>
-int launch_cond_prepare_kn(const CondPrepParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(kPredThreads), smem, scaml_cond_prepare_kernel<KIND, NJT>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml_cond_prepare_kernel<KIND, NJT>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_cond_prepare_kernel<KIND, NJT><<<grid, kPredThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-template <int KIND>
-int launch_cond_prepare_k(const CondPrepParams& p, int grid, size_t smem, void* stream) {
-  switch (p.pw) {
-    case 8: return launch_cond_prepare_kn<KIND, 1>(p, grid, smem, stream);
-    case 16: return launch_cond_prepare_kn<KIND, 2>(p, grid, smem, stream);
-    case 32: return launch_cond_prepare_kn<KIND, 4>(p, grid, smem, stream);
-    default: return launch_cond_prepare_kn<KIND, 8>(p, grid, smem, stream);
-  }
+  const int grid = p.M < 2 * num_sms ? p.M : 2 * num_sms;
+  return dispatch_kind(kernel, [&](auto K) {
+    return launch(scaml_cond_caches_kernel<K.value>, grid, 256, smem, stream, p);
+  });
 }
 
 inline int launch_cond_prepare(CondPrepParams p, int kernel, int num_sms, void* stream) {
@@ -487,43 +445,24 @@ inline int launch_cond_prepare(CondPrepParams p, int kernel, int num_sms, void* 
   const size_t smem = cond_prep_smem_bytes(p.n_pad, p.d, p.pw);
   long long items = (long long)p.M * p.npanel;
   int grid = (int)(items < num_sms ? items : num_sms);
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: return launch_cond_prepare_k<SCAML_KERNEL_RBF>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN12: return launch_cond_prepare_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream);
-    case SCAML_KERNEL_MATERN32: return launch_cond_prepare_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream);
-    default: return launch_cond_prepare_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream);
-  }
-}
-
-template <int KIND>
-int launch_cond_combine_k(const CondCombineParams& p, void* stream) {
-  const size_t smem = sizeof(double) * kCombTasks * (p.d + 1);
-  const long long pairs = (long long)p.B * p.n_t;
-  long long blocks = ((pairs + 255) / 256) * p.ntsplit;
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3((unsigned)(blocks < 2 ? blocks : 2)), dim3(256), smem, scaml_cond_combine_kernel<KIND>, p);
-  if (p.ntsplit > 1) cuemu::launch(dim3(1), dim3(256), 0, scaml_cond_combine_finish_kernel, p);
-  return 0;
-#else
-  if (blocks > 148 * 8) blocks = 148 * 8;
-  scaml_cond_combine_kernel<KIND><<<(int)blocks, 256, smem, (cudaStream_t)stream>>>(p);
-  int rc = (int)cudaGetLastError();
-  if (rc || p.ntsplit <= 1) return rc;
-  long long fb = (pairs + 255) / 256;
-  if (fb > 148 * 8) fb = 148 * 8;
-  scaml_cond_combine_finish_kernel<<<(int)fb, 256, 0, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
+  return dispatch_kind(kernel, [&](auto K) {
+    switch (p.pw) {
+      case 8: return launch(scaml_cond_prepare_kernel<K.value, 1>, grid, kPredThreads, smem, stream, p);
+      case 16: return launch(scaml_cond_prepare_kernel<K.value, 2>, grid, kPredThreads, smem, stream, p);
+      case 32: return launch(scaml_cond_prepare_kernel<K.value, 4>, grid, kPredThreads, smem, stream, p);
+      default: return launch(scaml_cond_prepare_kernel<K.value, 8>, grid, kPredThreads, smem, stream, p);
+    }
+  });
 }
 
 inline int launch_cond_combine(const CondCombineParams& p, int kernel, void* stream) {
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: return launch_cond_combine_k<SCAML_KERNEL_RBF>(p, stream);
-    case SCAML_KERNEL_MATERN12: return launch_cond_combine_k<SCAML_KERNEL_MATERN12>(p, stream);
-    case SCAML_KERNEL_MATERN32: return launch_cond_combine_k<SCAML_KERNEL_MATERN32>(p, stream);
-    default: return launch_cond_combine_k<SCAML_KERNEL_MATERN52>(p, stream);
-  }
+  const size_t smem = sizeof(double) * kCombTasks * (p.d + 1);
+  const long long blocks = (p.B * (long long)p.n_t + 255) / 256;
+  const int rc = dispatch_kind(kernel, [&](auto K) {
+    return launch(scaml_cond_combine_kernel<K.value>, stride_grid(blocks * p.ntsplit, 148 * 8), 256, smem, stream, p);
+  });
+  if (rc || p.ntsplit <= 1) return rc;
+  return launch(scaml_cond_combine_finish_kernel, stride_grid(blocks, 148 * 8), 256, 0, stream, p);
 }
 
 }  // namespace scaml

@@ -240,20 +240,6 @@ __global__ void scaml_cross_reduce_kernel(const double* part, double* cov, doubl
   }
 }
 
-template <int KIND>
-int launch_cross_k(const CrossParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(kFitThreads), smem, scaml_cross_kernel<KIND>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml_cross_kernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_cross_kernel<KIND><<<grid, kFitThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-
 inline size_t cross_workspace_bytes(int M, int nA, int nB, int reduce, int num_sms) {
   if (!reduce) return 0;
   const int tiles = ((nA + kCT - 1) / kCT) * ((nB + kCT - 1) / kCT);
@@ -278,24 +264,13 @@ inline int launch_predict_cross(const double* X, const int32_t* n_valid, const d
   long long items = reduce ? (long long)tiles * p.nsplit : (long long)tiles * M;
   long long cap = 4LL * num_sms;
   int grid = (int)(items < cap ? items : cap);
-  int rc;
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: rc = launch_cross_k<SCAML_KERNEL_RBF>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN12: rc = launch_cross_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN32: rc = launch_cross_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream); break;
-    default: rc = launch_cross_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream); break;
-  }
+  const int rc = dispatch_kind(kernel, [&](auto K) {
+    return launch(scaml_cross_kernel<K.value>, grid, kFitThreads, smem, stream, p);
+  });
   if (rc != 0 || !reduce || p.nsplit == 1) return rc;
   const long long ncov = (long long)nA * nB;
-#ifdef SCAML_EMU
-  cuemu::launch(dim3(1), dim3(64), 0, scaml_cross_reduce_kernel, (const double*)workspace, cov, mean, p.nsplit, ncov, nA);
-  return 0;
-#else
-  long long nb = (ncov + nA + 255) / 256;
-  scaml_cross_reduce_kernel<<<(int)(nb < 1184 ? nb : 1184), 256, 0, (cudaStream_t)stream>>>(workspace, cov, mean,
-                                                                                           p.nsplit, ncov, nA);
-  return (int)cudaGetLastError();
-#endif
+  return launch(scaml_cross_reduce_kernel, stride_grid((ncov + nA + 255) / 256, 1184), 256, 0, stream, workspace, cov,
+                mean, p.nsplit, ncov, nA);
 }
 
 }  // namespace scaml

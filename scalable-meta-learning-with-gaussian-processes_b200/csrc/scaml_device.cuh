@@ -1,5 +1,5 @@
-// Device-side helpers shared by the ScaML-GP kernels (sm_100a; also compiles under the
-// CPU logic emulation in emu/cuda_emu.h when SCAML_EMU is defined).
+// Device-side helpers shared by the ScaML-GP kernels, and the host-side launch and dispatch helpers (sm_100a; also
+// compiles under the CPU logic emulation in emu/cuda_emu.h when SCAML_EMU is defined).
 #pragma once
 
 #ifdef SCAML_EMU
@@ -19,6 +19,8 @@ inline double2 make_double2(double x, double y) { return double2{x, y}; }
 #endif
 
 #include <stdint.h>
+
+#include <type_traits>
 
 #include "../../include/scaml_b200.h"
 
@@ -349,5 +351,56 @@ SCAML_DEVICE double sigmoid(double x) { return 1.0 / (1.0 + exp(-x)); }
 
 // target points padded to whole 8-column DMMA blocks (shared by the conditioning and the gradient kernels)
 inline int cond_ntp(int n_t) { return ((n_t + 7) / 8) * 8; }
+
+// ----------------------------------------------------------------------------------- //
+// host side: every kernel launch and every choice of a kernel-family template
+// ----------------------------------------------------------------------------------- //
+// kern<<<grid, block, smem, stream>>>(args...) on the GPU, CTA by CTA on the CPU emulation; 0 or the CUDA error.
+// Dynamic shared memory above 48 KB needs the opt-in attribute.  It is per device and the sharded path drives several
+// GPUs from one process, so it is set on every such launch rather than cached.
+template <class... P, class... A>
+inline int launch(void (*kern)(P...), dim3 grid, dim3 block, size_t smem, void* stream, const A&... args) {
+#ifdef SCAML_EMU
+  (void)stream;
+  cuemu::launch(grid, block, smem, kern, args...);
+  return 0;
+#else
+  if (smem > 48 * 1024) {
+    const cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (err != cudaSuccess) return (int)err;
+  }
+  kern<<<grid, block, smem, (cudaStream_t)stream>>>(args...);
+  return (int)cudaGetLastError();
+#endif
+}
+
+// CTAs of a kernel that strides over `work` items by gridDim.x: at most gpu_cap on the GPU.  The emulation runs CTAs
+// one after another, so it runs two: enough to exercise the stride.
+inline int stride_grid(long long work, long long gpu_cap = INT32_MAX) {
+#ifdef SCAML_EMU
+  gpu_cap = 2;
+#endif
+  return (int)(work < gpu_cap ? work : gpu_cap);
+}
+
+// f(std::integral_constant<int, SCAML_KERNEL_*>) for the kernel-family id `kernel`; SCAML_E_ARG outside 0..3
+template <class F>
+inline int dispatch_kind(int kernel, F&& f) {
+  switch (kernel) {
+    case SCAML_KERNEL_RBF: return f(std::integral_constant<int, SCAML_KERNEL_RBF>());
+    case SCAML_KERNEL_MATERN12: return f(std::integral_constant<int, SCAML_KERNEL_MATERN12>());
+    case SCAML_KERNEL_MATERN32: return f(std::integral_constant<int, SCAML_KERNEL_MATERN32>());
+    case SCAML_KERNEL_MATERN52: return f(std::integral_constant<int, SCAML_KERNEL_MATERN52>());
+    default: return SCAML_E_ARG;
+  }
+}
+
+// f(std::integral_constant<int, DMAX>) for the kernels that keep per-dimension registers: DMAX = 8, 16 or 32 >= d
+template <class F>
+inline int dispatch_dmax(int d, F&& f) {
+  if (d <= 8) return f(std::integral_constant<int, 8>());
+  if (d <= 16) return f(std::integral_constant<int, 16>());
+  return f(std::integral_constant<int, 32>());
+}
 
 }  // namespace scaml

@@ -364,71 +364,29 @@ __global__ void __launch_bounds__(64) scaml_grad_finish_kernel(const GradParams 
   }
 }
 
-template <int KIND, int DMAX>
-int launch_grad_contract_kd(const GradParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(kGradThreads), smem, scaml_grad_contract_kernel<KIND, DMAX>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml_grad_contract_kernel<KIND, DMAX>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_grad_contract_kernel<KIND, DMAX><<<grid, kGradThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-template <int KIND>
-int launch_grad_contract_k(const GradParams& p, int grid, size_t smem, void* stream) {
-  if (p.d <= 8) return launch_grad_contract_kd<KIND, 8>(p, grid, smem, stream);
-  if (p.d <= 16) return launch_grad_contract_kd<KIND, 16>(p, grid, smem, stream);
-  return launch_grad_contract_kd<KIND, 32>(p, grid, smem, stream);
-}
-
 inline int launch_posterior_grad(GradParams p, int kernel, int num_sms, void* stream) {
   const size_t smem = grad_smem_bytes(p.n_pad, p.d, p.n_tp);
   if (smem > 227 * 1024) return SCAML_E_SMEM;
   if (p.n_t > 0) {
     const size_t msm = grad_mix_smem_bytes(p.n_tp, p.B_p);
     if (msm > 227 * 1024) return SCAML_E_SMEM;
-    const long long mitems = (long long)p.M * (p.n_pad / 32);
-#ifdef SCAML_EMU
-    cuemu::launch(dim3((unsigned)(mitems < 2 ? mitems : 2)), dim3(kGradThreads), msm, scaml_grad_mix_kernel, p);
-#else
     int per_sm = (int)((227 * 1024) / (msm + 1024));
     if (per_sm > 4) per_sm = 4;
     if (per_sm < 1) per_sm = 1;
-    const long long mg = mitems < (long long)per_sm * num_sms ? mitems : (long long)per_sm * num_sms;
-    cudaError_t merr = cudaFuncSetAttribute(scaml_grad_mix_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)msm);
-    if (merr != cudaSuccess) return (int)merr;
-    scaml_grad_mix_kernel<<<(unsigned)mg, kGradThreads, msm, (cudaStream_t)stream>>>(p);
-    merr = cudaGetLastError();
-    if (merr != cudaSuccess) return (int)merr;
-#endif
+    const long long mitems = (long long)p.M * (p.n_pad / 32);
+    const int rc = launch(scaml_grad_mix_kernel, stride_grid(mitems, (long long)per_sm * num_sms), kGradThreads, msm,
+                          stream, p);
+    if (rc) return rc;
   }
-  const int items = p.nsplit * p.ntile;
-#ifdef SCAML_EMU
-  const int grid = items < 2 ? items : 2;
-#else
-  const int grid = items < 2 * num_sms ? items : 2 * num_sms;
-#endif
-  int rc;
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: rc = launch_grad_contract_k<SCAML_KERNEL_RBF>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN12: rc = launch_grad_contract_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN32: rc = launch_grad_contract_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream); break;
-    default: rc = launch_grad_contract_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream); break;
-  }
+  const int grid = stride_grid(p.nsplit * p.ntile, 2 * num_sms);
+  const int rc = dispatch_kind(kernel, [&](auto K) {
+    return dispatch_dmax(p.d, [&](auto D) {
+      return launch(scaml_grad_contract_kernel<K.value, D.value>, grid, kGradThreads, smem, stream, p);
+    });
+  });
   if (rc) return rc;
-  long long gx = ((long long)p.B + 1) / 2;  // one warp per candidate, two warps per CTA
-#ifdef SCAML_EMU
-  cuemu::launch(dim3((unsigned)(gx < 2 ? gx : 2)), dim3(64), 0, scaml_grad_finish_kernel, p);
-  return 0;
-#else
-  if (gx > 4LL * num_sms) gx = 4LL * num_sms;
-  scaml_grad_finish_kernel<<<(unsigned)gx, 64, 0, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
+  // one warp per candidate, two warps per CTA
+  return launch(scaml_grad_finish_kernel, stride_grid(((long long)p.B + 1) / 2, 4LL * num_sms), 64, 0, stream, p);
 }
 
 }  // namespace scaml

@@ -191,54 +191,19 @@ inline int gradval_nsplit(int M, int ntile, int num_sms) {
   return ns < 1 ? 1 : ns;
 }
 
-template <int KIND, int NCB>
-int launch_grad_values_kn(const GradValParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(kGvThreads), smem, scaml_grad_values_kernel<KIND, NCB>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml_grad_values_kernel<KIND, NCB>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_grad_values_kernel<KIND, NCB><<<grid, kGvThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-template <int KIND>
-int launch_grad_values_k(const GradValParams& p, int grid, size_t smem, void* stream) {
-  const int ncb = p.n_tp / 8 + 1;  // accumulator column blocks per warp: register variants 5 / 9 / 17
-  if (ncb <= 5) return launch_grad_values_kn<KIND, 5>(p, grid, smem, stream);
-  if (ncb <= 9) return launch_grad_values_kn<KIND, 9>(p, grid, smem, stream);
-  return launch_grad_values_kn<KIND, kGvMaxCB>(p, grid, smem, stream);
-}
-
 inline int launch_grad_values(const GradValParams& p, int kernel, int num_sms, void* stream) {
   const size_t smem = gradval_smem_bytes(p.d, p.n_tp);
   if (smem > 227 * 1024) return SCAML_E_SMEM;
-  const int items = p.nsplit * p.ntile;
-#ifdef SCAML_EMU
-  const int grid = items < 2 ? items : 2;
-#else
-  const int grid = items < 4 * num_sms ? items : 4 * num_sms;
-#endif
-  int rc;
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: rc = launch_grad_values_k<SCAML_KERNEL_RBF>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN12: rc = launch_grad_values_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN32: rc = launch_grad_values_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream); break;
-    default: rc = launch_grad_values_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream); break;
-  }
+  const int grid = stride_grid(p.nsplit * p.ntile, 4 * num_sms);
+  const int ncb = p.n_tp / 8 + 1;  // accumulator column blocks per warp: register variants 5 / 9 / 17
+  const int rc = dispatch_kind(kernel, [&](auto K) {
+    if (ncb <= 5) return launch(scaml_grad_values_kernel<K.value, 5>, grid, kGvThreads, smem, stream, p);
+    if (ncb <= 9) return launch(scaml_grad_values_kernel<K.value, 9>, grid, kGvThreads, smem, stream, p);
+    return launch(scaml_grad_values_kernel<K.value, kGvMaxCB>, grid, kGvThreads, smem, stream, p);
+  });
   if (rc) return rc;
-  long long gx = ((long long)p.B + 1) / 2;
-#ifdef SCAML_EMU
-  cuemu::launch(dim3((unsigned)(gx < 2 ? gx : 2)), dim3(64), 0, scaml_grad_values_finish_kernel, p);
-  return 0;
-#else
-  if (gx > 4LL * num_sms) gx = 4LL * num_sms;
-  scaml_grad_values_finish_kernel<<<(unsigned)gx, 64, 0, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
+  const int fgrid = stride_grid(((long long)p.B + 1) / 2, 4LL * num_sms);  // one warp per candidate, two per CTA
+  return launch(scaml_grad_values_finish_kernel, fgrid, 64, 0, stream, p);
 }
 
 }  // namespace scaml

@@ -392,27 +392,6 @@ __global__ void __launch_bounds__(256, 3) scaml_kmat_task_kernel(const KmatParam
   }
 }
 
-template <int KIND>
-int launch_kmat_k(const KmatParams& p, int grid, size_t smem, bool task, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  if (task) cuemu::launch(dim3(grid), dim3(256), smem, scaml_kmat_task_kernel<KIND>, p);
-  else cuemu::launch(dim3(grid), dim3(256), smem, scaml_kmat_tile_kernel<KIND>, p);
-  return 0;
-#else
-  if (smem > 48 * 1024) {
-    cudaError_t err = task ? cudaFuncSetAttribute(scaml_kmat_task_kernel<KIND>,
-                                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                           : cudaFuncSetAttribute(scaml_kmat_tile_kernel<KIND>,
-                                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (err != cudaSuccess) return (int)err;
-  }
-  if (task) scaml_kmat_task_kernel<KIND><<<grid, 256, smem, (cudaStream_t)stream>>>(p);
-  else scaml_kmat_tile_kernel<KIND><<<grid, 256, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-
 // variant: 0 = by shape (whole-task kernel when the task's scaled inputs fit kKTaskSmem), 1 = tile kernel, 2 = task kernel
 inline int launch_kmat(const double* X, const int32_t* n_valid, const double* theta, double* K, int M, int n_max,
                        int d, int kernel, void* stream, int variant = 0) {
@@ -424,18 +403,11 @@ inline int launch_kmat(const double* X, const int32_t* n_valid, const double* th
   const bool task = (variant == 2) || (variant == 0 && tsmem <= kKTaskSmem);
   if (task && tsmem > 227 * 1024) return SCAML_E_SMEM;
   const size_t smem = task ? tsmem : kmat_smem_bytes(d);
-  long long g = task ? (long long)M : p.items;
-#ifdef SCAML_EMU
-  if (g > 4) g = 4;
-#else
-  if (g > 148LL * 8 * 4) g = 148LL * 8 * 4;
-#endif
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: return launch_kmat_k<SCAML_KERNEL_RBF>(p, (int)g, smem, task, stream);
-    case SCAML_KERNEL_MATERN12: return launch_kmat_k<SCAML_KERNEL_MATERN12>(p, (int)g, smem, task, stream);
-    case SCAML_KERNEL_MATERN32: return launch_kmat_k<SCAML_KERNEL_MATERN32>(p, (int)g, smem, task, stream);
-    default: return launch_kmat_k<SCAML_KERNEL_MATERN52>(p, (int)g, smem, task, stream);
-  }
+  const int grid = stride_grid(task ? (long long)M : p.items, 148LL * 8 * 4);
+  return dispatch_kind(kernel, [&](auto K) {
+    return task ? launch(scaml_kmat_task_kernel<K.value>, grid, 256, smem, stream, p)
+                : launch(scaml_kmat_tile_kernel<K.value>, grid, 256, smem, stream, p);
+  });
 }
 
 }  // namespace scaml

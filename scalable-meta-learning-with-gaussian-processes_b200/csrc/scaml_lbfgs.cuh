@@ -317,16 +317,8 @@ inline int launch_lbfgs_step(const LbfgsParams& p, void* stream) {
   const bool wide = p.D >= kLbWideMinD;  // by shape only: the reduction order of a row never depends on the batch
   const int grid = wide ? p.E : (p.E + kLbWarps - 1) / kLbWarps;
   const size_t smem = sizeof(double) * (wide ? (kLbMaxHistory + kLbWideWarps) : kLbWarps * (kLbMaxHistory + 1));
-#ifdef SCAML_EMU
-  (void)stream;
-  if (wide) cuemu::launch(dim3(grid), dim3(kLbWideWarps * 32), smem, scaml_lbfgs_step_kernel<kLbWideWarps>, p);
-  else cuemu::launch(dim3(grid), dim3(kLbWarps * 32), smem, scaml_lbfgs_step_kernel<1>, p);
-  return 0;
-#else
-  if (wide) scaml_lbfgs_step_kernel<kLbWideWarps><<<grid, kLbWideWarps * 32, smem, (cudaStream_t)stream>>>(p);
-  else scaml_lbfgs_step_kernel<1><<<grid, kLbWarps * 32, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
+  if (wide) return launch(scaml_lbfgs_step_kernel<kLbWideWarps>, grid, kLbWideWarps * 32, smem, stream, p);
+  return launch(scaml_lbfgs_step_kernel<1>, grid, kLbWarps * 32, smem, stream, p);
 }
 
 }  // namespace scaml

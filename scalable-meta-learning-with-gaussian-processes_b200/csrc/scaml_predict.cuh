@@ -720,29 +720,6 @@ __global__ void __launch_bounds__(128) scaml_predict_reduce_wide_kernel(const do
   }
 }
 
-template <int KIND, int CT, bool CROSS>
-int launch_predict_kc(const PredParams& p, int grid, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid), dim3(kPredThreads), smem, scaml_predict_kernel<KIND, CT, CROSS>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml_predict_kernel<KIND, CT, CROSS>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_predict_kernel<KIND, CT, CROSS><<<grid, kPredThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-template <int KIND>
-int launch_predict_k(const PredParams& p, int grid, size_t smem, void* stream) {
-  if (p.condA != nullptr)
-    return p.ct == 64 ? launch_predict_kc<KIND, 64, true>(p, grid, smem, stream)
-                      : launch_predict_kc<KIND, 32, true>(p, grid, smem, stream);
-  return p.ct == 64 ? launch_predict_kc<KIND, 64, false>(p, grid, smem, stream)
-                    : launch_predict_kc<KIND, 32, false>(p, grid, smem, stream);
-}
-
 // condA != null: also accumulate the cross-covariance partials into cxp (needs 64-candidate tiles: SCAML_E_SMEM
 // otherwise); workspace layout: [nsplit][2][B] mean/var partials (nsplit > 1) -- cxp is a separate buffer
 inline int launch_predict_weighted(const double* X, const int32_t* n_valid, const double* theta, const double* linv,
@@ -762,31 +739,19 @@ inline int launch_predict_weighted(const double* X, const int32_t* n_valid, cons
   const size_t smem = predict_smem_bytes(n_pad, d, p.ct, p.alias);
   long long items = (long long)p.ntile * p.nsplit;
   int grid = (int)(items < num_sms ? items : num_sms);
-  int rc;
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: rc = launch_predict_k<SCAML_KERNEL_RBF>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN12: rc = launch_predict_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN32: rc = launch_predict_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream); break;
-    default: rc = launch_predict_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream); break;
-  }
+  const int rc = dispatch_kind(kernel, [&](auto K) {
+    if (condA != nullptr)
+      return p.ct == 64 ? launch(scaml_predict_kernel<K.value, 64, true>, grid, kPredThreads, smem, stream, p)
+                        : launch(scaml_predict_kernel<K.value, 32, true>, grid, kPredThreads, smem, stream, p);
+    return p.ct == 64 ? launch(scaml_predict_kernel<K.value, 64, false>, grid, kPredThreads, smem, stream, p)
+                      : launch(scaml_predict_kernel<K.value, 32, false>, grid, kPredThreads, smem, stream, p);
+  });
   if (rc != 0 || p.nsplit == 1) return rc;
-  const bool wide = p.nsplit >= 32;  // by shape only
-#ifdef SCAML_EMU
-  if (wide) cuemu::launch(dim3(1), dim3(128), 0, scaml_predict_reduce_wide_kernel, (const double*)workspace, mean, var, p.nsplit, B);
-  else cuemu::launch(dim3(1), dim3(64), 0, scaml_predict_reduce_kernel, (const double*)workspace, mean, var, p.nsplit, B);
-  return 0;
-#else
-  if (wide) {
-    const int wb = (B + 3) / 4;
-    scaml_predict_reduce_wide_kernel<<<wb < 1184 ? wb : 1184, 128, 0, (cudaStream_t)stream>>>(workspace, mean, var,
-                                                                                             p.nsplit, B);
-  } else {
-    const int rb = (B + 255) / 256;
-    scaml_predict_reduce_kernel<<<rb < 1184 ? rb : 1184, 256, 0, (cudaStream_t)stream>>>(workspace, mean, var,
-                                                                                        p.nsplit, B);
-  }
-  return (int)cudaGetLastError();
-#endif
+  if (p.nsplit >= 32)  // by shape only
+    return launch(scaml_predict_reduce_wide_kernel, stride_grid((B + 3) / 4, 1184), 128, 0, stream, workspace, mean,
+                  var, p.nsplit, B);
+  return launch(scaml_predict_reduce_kernel, stride_grid((B + 255) / 256, 1184), 256, 0, stream, workspace, mean, var,
+                p.nsplit, B);
 }
 
 }  // namespace scaml

@@ -304,74 +304,38 @@ __global__ void __launch_bounds__(64) scaml_qblock_direct_kernel(const QBlockVjp
   }
 }
 
-template <typename Params>
-inline int qblock_launch(void (*kern)(Params), int grid, int threads, size_t smem, const Params& p, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(grid < 2 ? grid : 2), dim3(threads), smem, kern, p);
-  return 0;
-#else
-  if (smem > 48 * 1024) {
-    cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (err != cudaSuccess) return (int)err;
-  }
-  kern<<<grid, threads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-
-template <int KIND>
-int launch_qblock_cov_k(const QBlockCovParams& p, int grid, size_t smem, void* stream) {
-  if (p.d <= 8) return qblock_launch(scaml_qblock_cov_kernel<KIND, 8>, grid, kQbThreads, smem, p, stream);
-  if (p.d <= 16) return qblock_launch(scaml_qblock_cov_kernel<KIND, 16>, grid, kQbThreads, smem, p, stream);
-  return qblock_launch(scaml_qblock_cov_kernel<KIND, 32>, grid, kQbThreads, smem, p, stream);
-}
-
 inline int launch_qblock_cov(const QBlockCovParams& p, int kernel, int num_sms, void* stream) {
   const size_t smem = qblock_cov_smem_bytes(p.n_pad, p.d);
   if (smem > 227 * 1024) return SCAML_E_SMEM;
-  const int items = p.nsplit * p.ntile;
-  const int grid = items < 2 * num_sms ? items : 2 * num_sms;
-  int rc;
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: rc = launch_qblock_cov_k<SCAML_KERNEL_RBF>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN12: rc = launch_qblock_cov_k<SCAML_KERNEL_MATERN12>(p, grid, smem, stream); break;
-    case SCAML_KERNEL_MATERN32: rc = launch_qblock_cov_k<SCAML_KERNEL_MATERN32>(p, grid, smem, stream); break;
-    default: rc = launch_qblock_cov_k<SCAML_KERNEL_MATERN52>(p, grid, smem, stream); break;
-  }
+  const int grid = stride_grid(p.nsplit * p.ntile, 2 * num_sms);
+  const int rc = dispatch_kind(kernel, [&](auto K) {
+    return dispatch_dmax(p.d, [&](auto D) {
+      return launch(scaml_qblock_cov_kernel<K.value, D.value>, grid, kQbThreads, smem, stream, p);
+    });
+  });
   if (rc) return rc;
-  const long long n = (long long)p.B * p.q;
-  return qblock_launch(scaml_qblock_cov_finish_kernel, (int)((n + 127) / 128), 128, 0, p, stream);
-}
-
-template <int KIND>
-int launch_qblock_direct_k(const QBlockVjpParams& p, int grid, void* stream) {
-  if (p.d <= 8) return qblock_launch(scaml_qblock_direct_kernel<KIND, 8>, grid, 64, 0, p, stream);
-  if (p.d <= 16) return qblock_launch(scaml_qblock_direct_kernel<KIND, 16>, grid, 64, 0, p, stream);
-  return qblock_launch(scaml_qblock_direct_kernel<KIND, 32>, grid, 64, 0, p, stream);
+  return launch(scaml_qblock_cov_finish_kernel, stride_grid(((long long)p.B * p.q + 127) / 128), 128, 0, stream, p);
 }
 
 // fold, then the q = 1 gradient path on the folded inputs (g.beta = beta~, g.dmean / g.dvar the intermediate
 // outputs), then the direct terms and the combination
 inline int launch_qblock_vjp(const QBlockVjpParams& p, GradParams g, int kernel, int num_sms, void* stream) {
   const long long fitems = (long long)p.M * (p.n_pad / 32);
-  int rc = qblock_launch(scaml_qblock_fold_kernel, (int)(fitems < 4LL * num_sms ? fitems : 4LL * num_sms),
-                         kFoldThreads, qblock_fold_smem_bytes(p.B_p), p, stream);
+  int rc = launch(scaml_qblock_fold_kernel, stride_grid(fitems, 4LL * num_sms), kFoldThreads,
+                  qblock_fold_smem_bytes(p.B_p), stream, p);
   if (rc) return rc;
   if (p.n_t > 0) {
-    const long long n = (long long)p.B * p.n_tp;
-    rc = qblock_launch(scaml_qblock_fold_beta_kernel, (int)((n + 127) / 128), 128, 0, p, stream);
+    rc = launch(scaml_qblock_fold_beta_kernel, stride_grid(((long long)p.B * p.n_tp + 127) / 128), 128, 0, stream, p);
     if (rc) return rc;
   }
   rc = launch_posterior_grad(g, kernel, num_sms, stream);
   if (rc) return rc;
-  const int grid = (p.B + 1) / 2;  // one warp per point, two per CTA
-  switch (kernel) {
-    case SCAML_KERNEL_RBF: return launch_qblock_direct_k<SCAML_KERNEL_RBF>(p, grid, stream);
-    case SCAML_KERNEL_MATERN12: return launch_qblock_direct_k<SCAML_KERNEL_MATERN12>(p, grid, stream);
-    case SCAML_KERNEL_MATERN32: return launch_qblock_direct_k<SCAML_KERNEL_MATERN32>(p, grid, stream);
-    default: return launch_qblock_direct_k<SCAML_KERNEL_MATERN52>(p, grid, stream);
-  }
+  const int grid = stride_grid((p.B + 1) / 2);  // one warp per point, two per CTA
+  return dispatch_kind(kernel, [&](auto K) {
+    return dispatch_dmax(p.d, [&](auto D) {
+      return launch(scaml_qblock_direct_kernel<K.value, D.value>, grid, 64, 0, stream, p);
+    });
+  });
 }
 
 }  // namespace scaml

@@ -394,99 +394,35 @@ __global__ void __launch_bounds__(kPostThreads) scaml_target_posterior_kernel(co
     }
   }
 }
-template <bool BIG>
-int launch_target_posterior_v(const TargetPostParams& p, size_t smem, long long gx, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(gx < 2 ? (unsigned)gx : 2u), dim3(kPostThreads), smem, scaml_target_posterior_kernel<BIG>, p);
-  return 0;
-#else
-  cudaError_t err =
-      cudaFuncSetAttribute(scaml_target_posterior_kernel<BIG>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_target_posterior_kernel<BIG><<<(unsigned)gx, kPostThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
 inline int launch_target_posterior(const TargetPostParams& p, int num_sms, void* stream) {
   size_t smem = target_post_smem_bytes(p.nt, p.d);
   const bool big = smem > 227 * 1024;
   if (big) smem -= sizeof(double) * (size_t)p.nt * (p.nt | 1);
   if (smem > 227 * 1024 || p.nt > kTgtMaxPoints) return SCAML_E_SMEM;
-  long long gx = ((long long)p.B + kPostThreads / 32 - 1) / (kPostThreads / 32);
-  if (gx > 2LL * num_sms) gx = 2LL * num_sms;
-  return big ? launch_target_posterior_v<true>(p, smem, gx, stream) : launch_target_posterior_v<false>(p, smem, gx, stream);
-}
-
-template <int KIND, bool BIG>
-int launch_target_factor_v(const TargetParams& p, size_t smem, void* stream) {
-#ifdef SCAML_EMU
-  (void)stream;
-  cuemu::launch(dim3(p.R), dim3(kTgtThreads), smem, scaml_target_factor_kernel<KIND, BIG>, p);
-  return 0;
-#else
-  cudaError_t err = cudaFuncSetAttribute(scaml_target_factor_kernel<KIND, BIG>,
-                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (err != cudaSuccess) return (int)err;
-  scaml_target_factor_kernel<KIND, BIG><<<p.R, kTgtThreads, smem, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
-}
-// smem = target_smem_bytes(nt, d) selects the shared-memory kernel, anything else (the BIG footprint) the global one
-template <int KIND>
-int launch_target_factor(const TargetParams& p, size_t smem, void* stream) {
-  if (smem == target_smem_bytes(p.nt, p.d)) return launch_target_factor_v<KIND, false>(p, smem, stream);
-  return launch_target_factor_v<KIND, true>(p, smem, stream);
+  const int grid = stride_grid(((long long)p.B + kPostThreads / 32 - 1) / (kPostThreads / 32), 2LL * num_sms);
+  return big ? launch(scaml_target_posterior_kernel<true>, grid, kPostThreads, smem, stream, p)
+             : launch(scaml_target_posterior_kernel<false>, grid, kPostThreads, smem, stream, p);
 }
 
 inline int launch_target(const TargetParams& p, int num_sms, void* stream) {
   size_t smem = target_smem_bytes(p.nt, p.d);
-  if (smem > 227 * 1024) {  // K, L^-1 and the scaled inputs move to the per-row global block
+  const bool big = smem > 227 * 1024;
+  if (big) {  // K, L^-1 and the scaled inputs move to the per-row global block
     if (p.nt < kTgtBigFrom || p.nt > kTgtMaxPoints || p.big == nullptr) return SCAML_E_SMEM;
     smem = target_big_smem_bytes(p.nt);
   }
   const long long items = (long long)p.nt * p.nt + p.nt;
-  long long gx = (items + 7) / 8;
-  if (gx > 8LL * num_sms) gx = 8LL * num_sms;
-  int gw = (p.M + kTgtThreads - 1) / kTgtThreads;
-#ifdef SCAML_EMU
-  (void)stream;
-  for (int r = 0; r < p.R; ++r) {  // the emulator runs 1-D grids: one row at a time
-    TargetParams q = p;
-    q.R = 1;
-    q.w += (size_t)r * p.M, q.theta_raw += (size_t)r * (p.d + 2), q.jitter = p.jitter ? p.jitter + r : nullptr;
-    q.lml += r, q.grad_theta += (size_t)r * (p.d + 2), q.info += r;
-    if (p.grad_w) q.grad_w += (size_t)r * p.M;
-    q.covw += (size_t)r * p.nt * p.nt, q.meanw += (size_t)r * p.nt, q.Wmat += (size_t)r * p.nt * p.nt,
-        q.alpha += (size_t)r * p.nt;
-    if (p.big) q.big += (size_t)r * target_big_doubles(p.nt);
-    cuemu::launch(dim3(2), dim3(kTgtThreads), 0, scaml_target_reduce_kernel, q);
-    int rc;
-    switch (p.spec.kernel) {
-      case SCAML_KERNEL_RBF: rc = launch_target_factor<SCAML_KERNEL_RBF>(q, smem, stream); break;
-      case SCAML_KERNEL_MATERN12: rc = launch_target_factor<SCAML_KERNEL_MATERN12>(q, smem, stream); break;
-      case SCAML_KERNEL_MATERN32: rc = launch_target_factor<SCAML_KERNEL_MATERN32>(q, smem, stream); break;
-      default: rc = launch_target_factor<SCAML_KERNEL_MATERN52>(q, smem, stream); break;
-    }
+  const dim3 reduce_grid(stride_grid((items + 7) / 8, 8LL * num_sms), p.R);
+  const dim3 wgrad_grid(stride_grid((p.M + kTgtThreads - 1) / kTgtThreads, 4LL * num_sms), p.R);
+  // the dispatch rejects an unknown kernel family before anything is launched
+  return dispatch_kind(p.spec.kernel, [&](auto K) {
+    int rc = launch(scaml_target_reduce_kernel, reduce_grid, kTgtThreads, 0, stream, p);
     if (rc) return rc;
-    if (p.grad_w != nullptr) cuemu::launch(dim3(gw < 2 ? gw : 2), dim3(kTgtThreads), 0, scaml_target_wgrad_kernel, q);
-  }
-  return 0;
-#else
-  scaml_target_reduce_kernel<<<dim3((unsigned)gx, p.R), kTgtThreads, 0, (cudaStream_t)stream>>>(p);
-  int rc = (int)cudaGetLastError();
-  if (rc) return rc;
-  switch (p.spec.kernel) {
-    case SCAML_KERNEL_RBF: rc = launch_target_factor<SCAML_KERNEL_RBF>(p, smem, stream); break;
-    case SCAML_KERNEL_MATERN12: rc = launch_target_factor<SCAML_KERNEL_MATERN12>(p, smem, stream); break;
-    case SCAML_KERNEL_MATERN32: rc = launch_target_factor<SCAML_KERNEL_MATERN32>(p, smem, stream); break;
-    default: rc = launch_target_factor<SCAML_KERNEL_MATERN52>(p, smem, stream); break;
-  }
-  if (rc || p.grad_w == nullptr) return rc;
-  if (gw > 4 * num_sms) gw = 4 * num_sms;
-  scaml_target_wgrad_kernel<<<dim3(gw, p.R), kTgtThreads, 0, (cudaStream_t)stream>>>(p);
-  return (int)cudaGetLastError();
-#endif
+    rc = big ? launch(scaml_target_factor_kernel<K.value, true>, p.R, kTgtThreads, smem, stream, p)
+             : launch(scaml_target_factor_kernel<K.value, false>, p.R, kTgtThreads, smem, stream, p);
+    if (rc || p.grad_w == nullptr) return rc;
+    return launch(scaml_target_wgrad_kernel, wgrad_grid, kTgtThreads, 0, stream, p);
+  });
 }
 
 }  // namespace scaml

@@ -3,7 +3,7 @@ any kernel is launched, or through the emulation engine)."""
 import pytest
 import torch
 
-from scamlgp_b200._capi import ScamlError, load_cuda_library
+from scamlgp_b200._capi import HyperSpec, ScamlError, load_cuda_library
 from scamlgp_b200.model import ScaMLGP, _compute_target_prior, meta_fit_scamlgp, significant_weights_mask
 from scamlgp_b200.modules import (GammaPrior, GaussianLikelihood, Interval, MaternKernel, ModelFittingError, RBFKernel,
                                   ScaleKernel, SupervisedDataset)
@@ -117,6 +117,23 @@ def test_model_errors_through_emulation(emu_engine):
     bad = {"a": SupervisedDataset(torch.rand(5, 2, dtype=DT), torch.full((5, 1), float("nan"), dtype=DT))}
     with pytest.raises(ModelFittingError, match="failed for all attempts"):
         meta_fit_scamlgp(bad, num_restarts_log_likelihood=1, seed=0, engine=emu_engine, fit_options=dict(maxiter=2))
+
+
+def test_target_entry_points_reject_an_unknown_kernel_family(emu_engine):
+    """The target-GP objective, its in-kernel jitter ladder and the target factorisation refuse a kernel family id
+    outside 0..3, like every other entry point, instead of running some other family."""
+    M, nt, d = 2, 3, 2
+    g = torch.Generator().manual_seed(3)
+    sm, sc = torch.rand(nt, M, dtype=DT, generator=g), torch.rand(nt, nt, M, dtype=DT, generator=g)
+    Xt, yt = torch.rand(nt, d, dtype=DT, generator=g), torch.rand(nt, dtype=DT, generator=g)
+    w, th = torch.ones(1, M, dtype=DT), torch.zeros(1, d + 2, dtype=DT)
+    spec = HyperSpec.target(kernel=4)
+    with pytest.raises(ScamlError, match="scaml_target_lml_grad: bad argument"):
+        emu_engine.target_lml_grad(sm, sc, Xt, yt, w, th, 0.0, 1.0, spec)
+    with pytest.raises(ScamlError, match="scaml_target_lml_grad_ladder: bad argument"):
+        emu_engine.target_lml_grad_safe(sm, sc, Xt, yt, w, th, 0.0, 1.0, spec)
+    with pytest.raises(ScamlError, match="scaml_target_factorize: bad argument"):
+        emu_engine.target_factorize(sm, sc, Xt, yt, w[0], th[0], 0.0, 1.0, spec)
 
 
 def test_acquisition_optimiser_falls_back_without_gradient_support():

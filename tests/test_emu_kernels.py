@@ -405,12 +405,16 @@ def _large_nt_case(eng, n_t, M=3, n=48, d=2, B=9):
     sm, sc = eng.predict_cross(fs, Xt.to(dev))
     assert float((sm.cpu() - cache.source_means).abs().max()) < TOL_MEAN_VAR * float(cache.source_means.abs().max())
     yt = cache.yt_std.to(dev).contiguous()
-    lml, gw, gt, info = eng.target_lml_grad_safe(sm, sc, Xt.to(dev), yt, w.reshape(1, -1).to(dev).contiguous(),
-                                                 th.reshape(1, -1).to(dev).contiguous(), cache.mu_all, cache.s_all, cspec)
-    v, ogw, ogt = _oracle_target_value_and_grads(cache, w, th, ospec)
-    assert int(info[0]) == 0 and abs(float(lml[0]) - v) < TOL_LML * abs(v)
-    assert np.abs(gw[0].cpu().numpy() - ogw).max() < TOL_GRAD * np.abs(ogw).max()
-    assert np.abs(gt[0].cpu().numpy() - ogt).max() < TOL_GRAD * max(np.abs(ogt).max(), np.abs(ogw).max())
+    g2 = torch.Generator().manual_seed(9)  # a second row with its own w and theta: per-row offsets of the global block
+    W = torch.stack([w, torch.rand(M, dtype=torch.float64, generator=g2) + 0.1])
+    TH = torch.stack([th, th + 0.3 * torch.randn(th.shape, dtype=torch.float64, generator=g2)])
+    lml, gw, gt, info = eng.target_lml_grad_safe(sm, sc, Xt.to(dev), yt, W.to(dev), TH.to(dev), cache.mu_all,
+                                                 cache.s_all, cspec)
+    for r in range(2):
+        v, ogw, ogt = _oracle_target_value_and_grads(cache, W[r], TH[r], ospec)
+        assert int(info[r]) == 0 and abs(float(lml[r]) - v) < TOL_LML * abs(v)
+        assert np.abs(gw[r].cpu().numpy() - ogw).max() < TOL_GRAD * np.abs(ogw).max()
+        assert np.abs(gt[r].cpu().numpy() - ogt).max() < TOL_GRAD * max(np.abs(ogt).max(), np.abs(ogw).max())
     ts = eng.target_factorize(sm, sc, Xt.to(dev), yt, w.to(dev), th.to(dev), cache.mu_all, cache.s_all, cspec)
     Xc = torch.rand(B, d, dtype=torch.float64, generator=g)
     pm, pv = eng.predict_weighted(fs, w.to(dev), Xc.to(dev))
